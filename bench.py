@@ -2,7 +2,7 @@
 """bench.py -- agent-days/sec of the per-day agent loop (BASELINE.json), measured on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload hus|varsinais|scenario:<name>|synth50m]
-                    [--replicas R | --total-seeds T] [--days D] [--impl reference]
+                    [--replicas R | --total-seeds T] [--days D] [--impl reference] [--dump-outputs DIR]
 
 Default workload `hus`: a "step" is one complete HUS run (1,685,983 agents x 180 days, the reference's default
 interventions; BASELINE configs[1]) of an ensemble of R seeds per GPU advanced by the same launches (configs[3]), every
@@ -17,6 +17,13 @@ max-over-ranks go through the same communicator.  No torch anywhere in this file
     --total-seeds T    T seeds in total, T / N per GPU (configs[3] as written: strong scaling)
     --workload varsinais | scenario:hammer-and-dance | scenario:mitigation | ...   the other ensemble configurations
     --workload synth50m  configs[4]: ONE synthetic 5e7-agent population, population-sharded over the N GPUs
+
+    --dump-outputs DIR what the timed path returned in its last timed step, as DIR/<name>.npy in float64: for the ensemble
+                       workloads moments_sum and moments_sumsq ([days, row], sums over all replicas of all ranks of each
+                       stats column and of its square) and n_replicas (0-d, the number of replicas summed); for synth50m
+                       series ([1, days, row], rank 0's int32 stats rows).  Every step's seeds follow from the arguments,
+                       so two builds run with the same arguments can be compared array for array.  Not available with
+                       --impl reference: that arm keeps only the timings of its runs, not their series.
 
 The default run also reports, beside the headline: the 256-total-seed strong-scaling point (N > 1), the synthetic
 50 M-agent population on the same N GPUs, the single-seed run, per-kernel device times in the production launch
@@ -269,7 +276,7 @@ def timed_ensemble(ctx, comm, days, steps, warmup, seed_of, sampler=None):
         ctx.run(days)                              # schedule H2D + the simulated days + sync
         dev_ms = eng.last_step_ms()                # CUDA events around the multi-day run only
         s1, s2, n = ctx.moments(0, days, reduce=True)      # the step's result: k_moments + ONE ncclAllReduce + D2H
-        return dev_ms, time.perf_counter() - t0
+        return dev_ms, time.perf_counter() - t0, dict(moments_sum=s1, moments_sumsq=s2, n_replicas=n)
 
     for step in range(warmup):
         one_step(step)
@@ -279,7 +286,7 @@ def timed_ensemble(ctx, comm, days, steps, warmup, seed_of, sampler=None):
     comm.barrier()
     dev_ms_total, wall_total = 0.0, 0.0
     for step in range(warmup, warmup + steps):
-        dev_ms, wall = one_step(step)
+        dev_ms, wall, outputs = one_step(step)
         dev_ms_total += dev_ms
         wall_total += wall
     comm.barrier()
@@ -288,11 +295,19 @@ def timed_ensemble(ctx, comm, days, steps, warmup, seed_of, sampler=None):
     dev_ms_total, wall_total = (float(x) for x in comm.allreduce(np.array([dev_ms_total, wall_total]), 'max'))
     s1, _ = eng.read_moments(0, days)              # this rank's curves of the last step: the algorithmic bytes are computed from them
     return dict(ms_per_step=dev_ms_total / steps, wall_per_step=wall_total / steps, s1=s1, h2d=(h1 - h0) / steps, d2h=(d1 - d0) / steps,
-                launches=launches, clocks=clocks)
+                launches=launches, clocks=clocks, outputs=outputs)
+
+
+def dump_outputs(directory, outputs):
+    """Write the last timed step's results as DIR/<name>.npy in float64, so that two builds can be compared value for value
+    (the seeds of every step are fixed by the arguments)."""
+    os.makedirs(directory, exist_ok=True)
+    for name, x in outputs.items():
+        np.save(os.path.join(directory, name + '.npy'), np.asarray(x, dtype=np.float64))
 
 
 def bench_synth(a, rank, world, local, n_agents, days, steps, warmup):
-    """configs[4]: one synthetic population sharded over the ranks.  -> dict for the JSON line (rank 0) / None."""
+    """configs[4]: one synthetic population sharded over the ranks.  -> (dict for the JSON line, the last step's results)."""
     from reina_b200 import comm as rcomm, sharded
     spec = sharded.shard_spec() if world > 1 else None
     ctx = make_synth_context(n_agents, local, days, spec)
@@ -318,7 +333,7 @@ def bench_synth(a, rank, world, local, n_agents, days, steps, warmup):
                exchange={0: 'none', 1: 'ncclAllGather', 2: 'NVLink peer memory'}[int(eng.lib.f['shard_exchange'](eng.h))],
                message_bytes_per_rank_per_day=int(eng.lib.f['shard_message_bytes'](eng.h)))
     ctx.close()
-    return out
+    return out, dict(series=rows)
 
 
 def main():
@@ -334,7 +349,14 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='headline only: no strong-scaling point, synthetic population, single seed')
     ap.add_argument('--dump-daily', default=None, help='write the per-day I_d, E_d (ensemble means) the algorithmic bytes are computed from')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write what the timed path returned in its last step as DIR/<name>.npy (float64): the ensemble moments '
+                         '(moments_sum, moments_sumsq, n_replicas), or the daily rows (series) of --workload synth50m')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs is not available with --impl reference')
 
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
@@ -349,7 +371,9 @@ def main():
     peak_gbs, peak_src = load_peaks()
 
     if a.workload == 'synth50m':
-        r = bench_synth(a, rank, world, local, N_SYNTH, D, a.steps, a.warmup)
+        r, outputs = bench_synth(a, rank, world, local, N_SYNTH, D, a.steps, a.warmup)
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, outputs)
         if rank == 0:
             bytes_run = None
             out = dict(metric='agent-days/sec (synthetic 50M, population-sharded)', value=r['value'], unit='agent-days/s', n_gpus=world,
@@ -375,6 +399,8 @@ def main():
     seed_of = lambda step: 1_000_000 * (rank + 1) + 1000 * step     # fresh seeds every step, distinct per rank
 
     res = timed_ensemble(ctx, comm, D, a.steps, a.warmup, seed_of, ClockSampler(local) if rank == 0 else None)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, res['outputs'])
     agent_days_step = float(N) * D * R * world
     ms_per_step = res['ms_per_step']
     value = agent_days_step / (ms_per_step / 1e3)
@@ -465,8 +491,7 @@ def main():
         c2.close()
     # ---------------- configs[4]: the synthetic 50 M population on the same GPUs ----------------
     if extras:
-        s = bench_synth(a, rank, world, local, N_SYNTH, D, 2, 1)
-        out['synth50m'] = s
+        out['synth50m'], _ = bench_synth(a, rank, world, local, N_SYNTH, D, 2, 1)
     # ---------------- single-seed run of the same configuration (latency-bound, reported beside) ----------------
     if extras and rank == 0 and R != 1:
         c1 = make_context(spec, 1, local, D, seed=1)

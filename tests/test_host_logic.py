@@ -307,6 +307,20 @@ def test_surface_equals_the_reference_module(oracle_lib):
             ctx.apply_intervention(inputs.Intervention('no-such-intervention', '2020-01-01'))
 
 
+@pytest.mark.parametrize('gold_name,area', [('varsinais_suomi_default_n256', 'Varsinais-Suomi'), ('hus_default_n256', 'HUS')])
+def test_day0_state_equals_the_stored_reference_rows(oracle_lib, gold_name, area):
+    """The day-0 half of the comparison above without the reference module: before the first iterate() nothing is
+    random, so generate_state() must give, in every series, the value the unmodified reference engine gave in all 256
+    seeds of its stored ensemble (tests/golden/make_golden.py)."""
+    from oracle import ref_harness
+    gold = np.load(os.path.join(helpers.ROOT, 'tests', 'golden', 'ref_ensemble_%s.npz' % gold_name))
+    assert list(gold['names']) == ref_harness.series_names() and (gold['std'][0] == 0).all()
+    ctx = helpers.make_context(oracle_lib, area=area, seed=3)
+    row = np.array(ref_harness.state_row(ctx.generate_state()))
+    bad = np.flatnonzero(row != gold['mean'][0])
+    assert not len(bad), [(gold['names'][k], row[k], gold['mean'][0, k]) for k in bad]
+
+
 # ---------------------------------------------------------------------------------------------------
 # round-2 host logic: intervention ordering, direct apply_intervention, input validation, job pruning
 # ---------------------------------------------------------------------------------------------------

@@ -3,9 +3,10 @@
 driven over `reina_b200.model` bound as `cythonsim.model` -- the one-line integration INTEGRATION.md section 1 describes --
 side by side with the same call over the unmodified Cython engine (oracle/_ref).
 
-Needs the reference tree, so these run in the build container only (skipped on the GPU box, where /root/reference does
-not exist); the engine under the shim is therefore the CPU oracle library, injected through the test-only `_library`
-seam.  The CUDA engine runs behind exactly the same Python surface (tests/test_gpu_*.py compare the two bit for bit).
+The live comparisons need the reference source tree ($REF) and skip where it is absent; the engine under the shim is the
+CPU oracle library, injected through the test-only `_library` seam.  The CUDA engine runs behind exactly the same Python
+surface (tests/test_gpu_*.py compare the two bit for bit).  The deterministic cells they compare are also checked without
+the reference tree, against the reference engine's own output stored in tests/golden.
 """
 import os
 import pickle
@@ -20,7 +21,9 @@ import helpers
 REF = os.environ.get('REF', '/root/reference')
 SHIM = os.path.join(helpers.ROOT, 'tests', 'ref_caller_shim.py')
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'calc')), reason='needs the reference tree')
+needs_reference_tree = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'calc')), reason='needs the reference tree')
+# the unmodified reference engine, Varsinais-Suomi with the default interventions, 256 seeds (tests/golden/make_golden.py)
+REF_GOLD = os.path.join(helpers.ROOT, 'tests', 'golden', 'ref_ensemble_varsinais_suomi_default_n256.npz')
 
 
 def _run(engine, out, days, area='Varsinais-Suomi', seed=3):
@@ -31,6 +34,7 @@ def _run(engine, out, days, area='Varsinais-Suomi', seed=3):
         return pickle.load(f)
 
 
+@needs_reference_tree
 def test_real_caller_over_the_shim_matches_the_reference_engine(tmp_path):
     from oracle import ref_harness
     if not ref_harness.available():
@@ -66,6 +70,7 @@ def test_real_caller_over_the_shim_matches_the_reference_engine(tmp_path):
     assert np.array_equal(ab.to_numpy(), adf2.to_numpy()) and ab.columns.equals(adf2.columns)
 
 
+@needs_reference_tree
 @pytest.mark.gpu
 def test_real_caller_over_the_cuda_shim(tmp_path):
     """Only where a GPU and the reference tree meet (never on the driver's boxes): the same call over the shipped module."""
@@ -75,3 +80,27 @@ def test_real_caller_over_the_cuda_shim(tmp_path):
     cols = [c for c in cuda['df'].columns if c != 'us_per_infected']
     assert np.array_equal(cuda['df'][cols].to_numpy(dtype=float), orac['df'][cols].to_numpy(dtype=float))
     assert np.array_equal(cuda['adf'].to_numpy(), orac['adf'].to_numpy())
+
+
+@pytest.mark.parametrize('engine', ['oracle', pytest.param('cuda', marks=pytest.mark.gpu)])
+def test_caller_frames_hold_the_reference_engine_cells(engine):
+    """The deterministic cells of the live comparison above, without the reference tree: this repo's caller
+    (reina_b200.simulation, same area, days and seed) over the CPU oracle and over the CUDA engine, against the output of
+    the unmodified reference engine stored in REF_GOLD.  There these cells take the same value in all 256 seeds."""
+    from reina_b200 import inputs, simulation
+    gold = np.load(REF_GOLD)
+    names = list(gold['names'])
+    days = 30
+    v = inputs.default_variables(simulation_days=days, area_name='Varsinais-Suomi', random_seed=3)
+    lib = helpers.oracle_library() if engine == 'oracle' else helpers.cuda_library()
+    df, adf = simulation.simulate_individuals(v, context=simulation.make_context(v, _library=lib))
+    assert df.shape == (days, 26) and adf.shape == (days, 12 * 9)
+    for col in ('total_icu_units', 'mobility_limitation', 'vaccinated'):
+        j = names.index(col)
+        assert (gold['std'][:days, j] == 0).all(), col
+        assert np.array_equal(df[col].to_numpy(dtype=float), gold['mean'][:days, j]), col
+    j = names.index('susceptible')
+    assert gold['std'][0, j] == 0 and df['susceptible'].iloc[0] == gold['mean'][0, j] == 479861
+    assert adf['susceptible'].iloc[0].sum() == 479861
+    # the imports of 2020-02-22 .. 03-15 (default interventions) took hold
+    assert df['all_infected'].iloc[-1] > 200 and df['susceptible'].iloc[-1] + df['all_infected'].iloc[-1] == 479861
