@@ -189,6 +189,25 @@ int rb_sample(rb_engine *e, int32_t what, int32_t age, int32_t severity, int32_t
  * this call. */
 int rb_rng_block(int32_t words, uint32_t key, const uint32_t *ctr, uint32_t *out);
 
+/* Transmission statistics of the state after the last completed rb_step, from the infection tree every run keeps (no
+ * reference counterpart: main.pyx only reports r = total_infections / total_infectors, which mixes infection days).
+ * Per replica one int32 row of rb_transmission_len entries, M = max_days + 1:
+ *   cohort_infected[M], cohort_offspring[M], cohort_open[M]   by infection day d: infected agents, the sum of their
+ *                                                             other_people_infected, those still INCUBATION / ILLNESS
+ *   offspring_hist[RB_TX_BINS]                                closed cases (neither INCUBATION nor ILLNESS) by
+ *                                                             min(other_people_infected, 64)
+ *   gi_hist[RB_TX_BINS]                                       agents with an infector by min(d - d(infector), 64)
+ *   group_closed[n_groups], group_offspring[n_groups]         closed cases and their offspring by age group
+ *   variant_closed[RB_MAX_VARIANTS], variant_offspring[RB_MAX_VARIANTS]   the same by variant
+ * Identical on every rank of a population-sharded simulation.  CUDA library only: the tests' CPU reference is the oracle
+ * plus these three entry points as plain loops (tests/oracle_transmission.c). */
+#define RB_TX_BINS 65        /* histogram bins 0..63 and ">= 64" */
+int32_t rb_transmission_len(rb_engine *e);   /* 3 (max_days + 1) + 2 RB_TX_BINS + 2 n_groups + 2 RB_MAX_VARIANTS */
+/* out[n_replicas][rb_transmission_len] */
+int rb_transmission_stats(rb_engine *e, int32_t *out);
+/* Infection day of every agent of one replica (-1 = never infected): with rb_read_agents' infector, the transmission tree. */
+int rb_read_infection_days(rb_engine *e, int32_t replica, int32_t *out);
+
 /* Parity/debug exports. */
 int rb_read_agents(rb_engine *e, int32_t replica, rb_agent *out);
 int rb_read_queue(rb_engine *e, int32_t replica, int32_t *out, int32_t cap, int32_t *n);   /* test queue, in order */

@@ -19,6 +19,7 @@ RB_MAX_IMPORT_CLASSES = 16
 RB_N_PLACES = 6
 RB_IOT_LEN = 21
 RB_N_TABLES = 6
+RB_TX_BINS = 65      # offspring / generation-interval histograms: bins 0..63 and ">= 64"
 
 ATTRS = ['susceptible', 'vaccinated', 'infected', 'all_infected', 'detected', 'all_detected',
          'in_icu', 'cum_icu', 'in_ward', 'dead', 'recovered', 'non_hospital_deaths', 'new_infections']
@@ -87,13 +88,15 @@ SYMBOLS = ['create', 'destroy', 'reset', 'set_initial_state', 'step_profiled', '
            'read_queue', 'read_available', 'last_step_ms', 'launch_count', 'last_error', 'rng_block']
 
 
-# population-sharded mode: exported by the CUDA library only (the sequential CPU oracle has no ranks)
+# transmission statistics from the infection tree; their CPU reference is test code (tests/oracle_transmission.c)
+TX_SYMBOLS = ['transmission_len', 'transmission_stats', 'read_infection_days']
+# exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes']
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -187,6 +190,19 @@ class Library:
             f['copied_bytes'].argtypes = [vp, C.c_int32]
             f['copied_bytes'].restype = C.c_int64
         self.f = f
+        if prefix == 'rb_':
+            self.bind_transmission()
+
+    def bind_transmission(self):
+        """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
+        to the CPU oracle calls this itself)."""
+        f, vp = self.f, C.c_void_p
+        for name in TX_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['transmission_len'].argtypes = [vp]
+        f['transmission_len'].restype = C.c_int32
+        f['transmission_stats'].argtypes = [vp, C.POINTER(C.c_int32)]
+        f['read_infection_days'].argtypes = [vp, C.c_int32, C.POINTER(C.c_int32)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -377,6 +393,18 @@ class Engine:
     def read_available(self, replica=0):
         out = np.zeros(2, dtype=np.int32)
         self.lib.check(self.lib.f['read_available'](self.h, replica, _ptr(out, C.c_int32)), 'read_available')
+        return out
+
+    def transmission_stats(self):
+        """[replica, rb_transmission_len] int32: the transmission tables of every replica (reina_b200.h)."""
+        out = np.empty((self.n_replicas, self.lib.f['transmission_len'](self.h)), dtype=np.int32)
+        self.lib.check(self.lib.f['transmission_stats'](self.h, _ptr(out, C.c_int32)), 'transmission_stats')
+        return out
+
+    def read_infection_days(self, replica=0):
+        """Infection day of every agent of one replica, -1 = never infected."""
+        out = np.empty(self.n_agents, dtype=np.int32)
+        self.lib.check(self.lib.f['read_infection_days'](self.h, replica, _ptr(out, C.c_int32)), 'read_infection_days')
         return out
 
     def last_step_ms(self):

@@ -16,6 +16,7 @@
 //   shard.cuh     population-sharded mode: k_publish / k_wait (per-day flags in NVLink peer memory) and k_merge, which
 //                 pulls and applies every rank's message of the day
 //   setup.cuh     set_initial_state, initialisation, contact-row guide, snapshot, ensemble moments, samplers
+//   transmission.cuh  k_transmission: cohort / offspring / generation-interval tables from the infection tree (not per day)
 //   this file     host side: engine handle, launch geometry, replica groups, CUDA graphs, NCCL binding (ensemble reduce,
 //                 sharded mode), the extern "C" entry points
 //
@@ -29,6 +30,7 @@
 #include "shard.cuh"
 #include "setup.cuh"
 #include "run.cuh"
+#include "transmission.cuh"
 
 // ================================================================ host side / C-ABI
 static thread_local char g_err[512];
@@ -86,6 +88,7 @@ struct rb_engine {
     uint32_t xepoch; uint32_t *d_xepoch;   // host copy / device word of Eng::xepoch
     cudaGraphExec_t sh_graph[2]; bool have_sh_graphs;      // population-sharded days (peer-memory exchange): 16 days / 1 day
     Ipc ipc; bool has_ipc;              // initial population condition, re-applied by rb_reset
+    int32_t *d_tx;                      // [R][rb_transmission_len] tables of rb_transmission_stats, allocated by its first call
 };
 
 // ---------------------------------------------------------------- NCCL, bound at run time
@@ -200,7 +203,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     rb_engine *e = new rb_engine();
     e->cfg = *cfg; e->day = 0; e->last_ms = 0; e->launches = 0; e->h2d_bytes = 0; e->d2h_bytes = 0; e->have_graphs = false; e->comm = nullptr; e->comm_rank = 0; e->comm_size = 1; e->sharded = false; e->merge_blocks = 1;
     e->has_ipc = false; e->h_stage = nullptr; e->n_stage = 0; e->n_groups = 1; e->wide_ctas = 1; e->n_peer_open = 0; e->launch_err = cudaSuccess; e->shard_timing = getenv("RB_SHARD_TIMING") != nullptr;
-    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false;
+    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr;
     { int lo = 0, hi = 0; CK(cudaDeviceGetStreamPriorityRange(&lo, &hi)); e->prio_high = hi; e->prio = (cfg->n_replicas >= 32 && cfg->n_replicas < 128) ? 1 : 0; if (const char *s = getenv("RB_PRIO")) e->prio = atoi(s); }
     CK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&e->ev0)); CK(cudaEventCreate(&e->ev1));
@@ -1232,6 +1235,49 @@ extern "C" int rb_read_agents(rb_engine *e, int32_t replica, rb_agent *out) {
         o->flags = (uint8_t)(((h & H_DET) ? 1 : 0) | ((h & H_QUEUED) ? 2 : 0) | ((h & H_INCL) ? 4 : 0) | ((h & H_LIST) ? 8 : 0));
         o->ward_days = (uint8_t)((cold[a] >> 16) & 255u); o->icu_days = (uint8_t)((cold[a] >> 24) & 255u);
     }
+    return 0;
+}
+
+// ---------------------------------------------------------------- transmission statistics (transmission.cuh)
+extern "C" int32_t rb_transmission_len(rb_engine *e) { return tx_layout(e->cfg.max_days, e->cfg.n_groups).len; }
+
+extern "C" int rb_transmission_stats(rb_engine *e, int32_t *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    const Eng &G = e->G;
+    const TxLayout L = tx_layout(G.max_days, G.n_groups);
+    const size_t bytes = sizeof(int32_t) * (size_t)G.R * L.len, smem = sizeof(int32_t) * (size_t)L.len;
+    if (!e->d_tx && dalloc(e, &e->d_tx, (size_t)G.R * L.len)) return 1;
+    // shared counts of one replica: beyond the default 48 KB only for a max_days above ~4000
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_transmission, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // every state change is written to `hot` at once; the flush adds the day counters, so that these tables describe the
+    // same `hot` that rb_read_agents / rb_save_state see
+    k_flush_lists<<<dim3(e->sweep_blocks, G.R), 256, 0, e->stream>>>(G);
+    CK(cudaMemsetAsync(e->d_tx, 0, bytes, e->stream));
+    int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+    // about two waves of 256-thread CTAs over all replicas, and no CTA without agents
+    const int per_rep = std::max(1, std::min((2 * sms * (2048 / TX_THREADS) + G.R - 1) / G.R, (G.N + TX_THREADS - 1) / TX_THREADS));
+    k_transmission<<<dim3(per_rep, G.R), TX_THREADS, smem, e->stream>>>(G, L, e->d_tx);
+    e->launches += 2;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, e->d_tx, bytes, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->d2h_bytes += (int64_t)bytes;
+    return 0;
+}
+
+extern "C" int rb_read_infection_days(rb_engine *e, int32_t replica, int32_t *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    const Eng &G = e->G;
+    if (replica < 0 || replica >= G.R) { snprintf(g_err, sizeof g_err, "bad replica"); return 1; }
+    k_flush_lists<<<dim3(e->sweep_blocks, G.R), 256, 0, e->stream>>>(G);
+    int32_t *d; CK(cudaMallocAsync(&d, sizeof(int32_t) * G.N, e->stream));
+    k_infection_days<<<(G.N + 255) / 256, 256, 0, e->stream>>>(G, replica, d);
+    e->launches += 2;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, d, sizeof(int32_t) * G.N, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaFreeAsync(d, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->d2h_bytes += (int64_t)sizeof(int32_t) * G.N;
     return 0;
 }
 

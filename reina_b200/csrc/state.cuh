@@ -89,7 +89,7 @@ struct Attempt { uint32_t cand, parent; unsigned long long key; };
 struct __align__(32) AgentRec {
     unsigned long long winner;       // atomicMin conflict slot, all-ones when idle
     int32_t infector, first_child, next_sib;   // infection tree (replaces the malloc'd infectees[64], main.pyx:227-233)
-    uint32_t inf_key;                // (day << 8) | slot of this agent's infection: orders siblings
+    uint32_t inf_key;                // (day << 8) | slot of this agent's infection: orders siblings; day << 8 for a root
     uint32_t cold;                   // other_people_infected 16b | ward_days 8b | icu_days 8b
     int16_t vacc_day, pad;
 };
@@ -309,6 +309,8 @@ __device__ void device_infect(const Eng &G, int r, RepCtr *c, int32_t t, int32_t
         if ((src_h & H_LIST) && (old & 0xffffu) >= MAX_INFECTEES) set_problem(c, RB_TOO_MANY_INFECTEES);
         G.rec[base + t].inf_key = ((uint32_t)day << 8) | (uint32_t)slot;
         G.rec[base + t].next_sib = prev_child;
+    } else {
+        G.rec[base + t].inf_key = (uint32_t)day << 8;   // roots (imports, initial state) keep their infection day too: k_transmission
     }
     // a SUSCEPTIBLE agent's word carries nothing but the vaccinated flag, which vacc_day implies
     uint32_t nh = (vd >= 0 ? H_VACC : 0u) | RB_INCUBATION | ((uint32_t)sev << 3) | ((uint32_t)variant << 8) | ((uint32_t)dl << 14);

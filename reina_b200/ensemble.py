@@ -76,3 +76,59 @@ def run_ensemble(make_context, days, replicas_per_rank, seed0=0, comm=None):
         s1, s2, n = reduce_moments(*ctx.moments(0, days), comm=comm)
     mean, std = mean_std(s1, s2, n)
     return dict(mean=mean, std=std, n=n, names=ctx.row_layout(), context=ctx, comm=comm)
+
+
+_TX_SUMS = ('offspring_hist', 'generation_interval_hist', 'group_closed', 'group_offspring', 'variant_closed',
+            'variant_offspring')
+
+
+def transmission_summary(stats, comm=None):
+    """Ensemble transmission statistics from Context.transmission_stats() of every rank (one allreduce, like
+    reduce_moments).  With K the total number of replicas, n_r[d] / off_r[d] the infected / offspring of cohort d in
+    replica r:
+
+      cohort_R[d]      sum off / sum n, the ratio estimator of the cohort reproduction number (NaN where sum n = 0)
+      cohort_R_se[d]   its between-replica standard error by the delta method,
+                       SE^2 = sum_r (off_r - R n_r)^2 / (nbar^2 K (K - 1)), nbar = sum n / K
+      complete[d]      no agent of the cohort can infect any more (sum open == 0); later cohorts are right-censored
+      offspring_mean, offspring_var, dispersion_k   of the closed cases' offspring (bin 64 counts as 64);
+                       k = m^2 / (v - m), inf when v <= m (no overdispersion)
+      gi_pmf[k], gi_mean                            generation-interval distribution in days
+      R_by_group[g], R_by_variant[v]                offspring per closed case
+    plus the summed tables and K."""
+    comm = comm or LocalComm()
+    n = np.asarray(stats['cohort_infected'], dtype=np.float64)
+    off = np.asarray(stats['cohort_offspring'], dtype=np.float64)
+    parts = [n.sum(0), off.sum(0), (off * off).sum(0), (off * n).sum(0), (n * n).sum(0),
+             np.asarray(stats['cohort_open'], dtype=np.float64).sum(0)]
+    parts += [np.asarray(stats[k], dtype=np.float64).sum(0) for k in _TX_SUMS]
+    flat = np.concatenate(parts + [[float(n.shape[0])]])
+    if comm.size > 1:
+        flat = comm.allreduce(flat, 'sum')
+    out, k = {}, 0
+    for name, p in zip(('n', 'off', 'off2', 'offn', 'n2', 'open') + _TX_SUMS, parts):
+        out[name] = flat[k:k + p.size]
+        k += p.size
+    K = int(round(flat[-1]))
+    sn, so = out.pop('n'), out.pop('off')
+    s2, sxn, sn2 = out.pop('off2'), out.pop('offn'), out.pop('n2')
+    with np.errstate(divide='ignore', invalid='ignore'):
+        R = np.where(sn > 0, so / sn, np.nan)
+        nbar = sn / K
+        ss = np.maximum(s2 - 2.0 * R * sxn + R * R * sn2, 0.0)
+        se = np.sqrt(ss / (nbar * nbar * K * (K - 1))) if K > 1 else np.full_like(R, np.nan)
+        se = np.where(sn > 0, se, np.nan)
+        h = out['offspring_hist']
+        kk = np.arange(h.size, dtype=np.float64)
+        nc = h.sum()
+        m = (kk * h).sum() / nc if nc > 0 else np.nan
+        v = (((kk - m) ** 2) * h).sum() / (nc - 1) if nc > 1 else np.nan
+        disp = m * m / (v - m) if v > m else np.inf
+        g = out['generation_interval_hist']
+        pmf = g / g.sum() if g.sum() > 0 else np.full_like(g, np.nan)
+        r_group = np.where(out['group_closed'] > 0, out['group_offspring'] / out['group_closed'], np.nan)
+        r_var = np.where(out['variant_closed'] > 0, out['variant_offspring'] / out['variant_closed'], np.nan)
+    return dict(n_replicas=K, cohort_infected=sn, cohort_offspring=so, cohort_open=out['open'], cohort_R=R,
+                cohort_R_se=se, complete=out['open'] == 0, offspring_mean=m, offspring_var=v, dispersion_k=disp,
+                gi_pmf=pmf, gi_mean=float((np.arange(pmf.size) * pmf).sum()), R_by_group=r_group, R_by_variant=r_var,
+                **{name: out[name] for name in _TX_SUMS})

@@ -304,6 +304,8 @@ class Context:
             self._engine.shard_init(int(shard[0]), int(shard[1]), shard[2], float(shard[3]) if len(shard) > 3 else 0.0)
 
         self.n_agents, self.n_ages, self.n_replicas = n_agents, n_ages, int(n_replicas)
+        self._group_of_age = group_of_age[:n_ages].copy()
+        self._age_start = np.concatenate([[0], np.cumsum(age_counts)])      # agents are stored age-sorted
         self.max_days = int(max_days)
         self.start_date = start_date
         self.day = 0
@@ -484,6 +486,46 @@ class Context:
             return self._engine.reduce_moments(day0, days)
         s1, s2 = self._engine.read_moments(day0, days)
         return s1, s2, self.n_replicas
+
+    def transmission_stats(self):
+        """Who infected whom and when, per replica, from the infection tree of the current state (k_transmission; all
+        arrays int64 with a leading replica axis):
+
+          cohort_infected[r, d]    agents infected on day d, d = 0 .. today
+          cohort_offspring[r, d]   the people those agents have infected so far
+          cohort_open[r, d]        those agents still incubating or ill, i.e. still able to infect: while it is not 0 the
+                                   cohort's offspring count can grow (right-censored)
+          offspring_hist[r, k]     closed cases (no longer able to infect) that infected k people; k = 64 means >= 64
+          generation_interval_hist[r, k]   infected agents whose infector was infected k days earlier (64: >= 64)
+          group_closed / group_offspring[r, g]       closed cases and their offspring by age group (age_group_labels)
+          variant_closed / variant_offspring[r, v]   the same by variant (variant_names)
+
+        ensemble.transmission_summary() turns these into cohort reproduction numbers, dispersion and the
+        generation-interval distribution."""
+        t = self._engine.transmission_stats().astype(np.int64)
+        M, B, G, V = self.max_days + 1, _abi.RB_TX_BINS, len(self.age_group_labels), _abi.RB_MAX_VARIANTS
+        parts, k = {}, 0
+        for name, n in (('cohort_infected', M), ('cohort_offspring', M), ('cohort_open', M), ('offspring_hist', B),
+                        ('generation_interval_hist', B), ('group_closed', G), ('group_offspring', G),
+                        ('variant_closed', V), ('variant_offspring', V)):
+            parts[name] = t[:, k:k + n]
+            k += n
+        assert k == t.shape[1]
+        for name in ('cohort_infected', 'cohort_offspring', 'cohort_open'):
+            parts[name] = parts[name][:, :self.day + 1]
+        for name in ('variant_closed', 'variant_offspring'):
+            parts[name] = parts[name][:, :len(self.variant_names)]
+        return parts
+
+    def transmission_tree(self, replica=0):
+        """The line list of one replica: every agent infected so far, as arrays agent (index), infector (-1 for imports
+        and the initial state), day (of infection) and age."""
+        days = self._engine.read_infection_days(replica)
+        agent = np.flatnonzero(days >= 0)
+        infector = self._engine.read_agents(replica)['infector'][agent]
+        age = np.searchsorted(self._age_start, agent, side='right') - 1
+        return dict(agent=agent.astype(np.int64), infector=infector.astype(np.int64), day=days[agent].astype(np.int64),
+                    age=age.astype(np.int64))
 
     def row_layout(self):
         G = len(self.age_group_labels)

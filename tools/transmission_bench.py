@@ -1,0 +1,86 @@
+#!/usr/bin/env python
+"""Cost of Context.transmission_stats() at the bench geometry: full HUS (1,685,983 agents), 256 replicas, after a 180-day
+run with the default interventions.
+
+    python tools/transmission_bench.py [--replicas 256] [--days 180] [--calls 30] [--out FILE]
+
+Prints one JSON line: ms per call (host clock around the call, which ends in a stream synchronise), the byte model of
+k_transmission over that time as a share of the measured HBM bandwidth, and the ratio to the time of the 180-day run
+itself (last_step_ms).  The card's name and power limit are read in the same process.
+
+Byte model per replica (what the pass has to move at least): the susceptibility bitmap (N / 8 bytes), and per infected
+agent its 4-byte packed word and its 32-byte agent record, plus one gathered 32-byte record of the infector for every
+agent that has one.  The call also runs k_flush_lists (reads the active lists) and copies the tables to the host; both
+are inside the measured time and outside the byte model.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+HBM_GBS = 6456.2     # HBM bandwidth measured on a B200 (the peak of bench.py's roofline, profiles/r02_bench_R256_n1.json)
+
+
+def card():
+    try:
+        q = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader'],
+                           capture_output=True, text=True, timeout=30)
+        return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else 'unknown'
+    except (OSError, subprocess.SubprocessError):
+        return 'unknown'
+
+
+def byte_model(stats, n_agents):
+    infected = stats['cohort_infected'].sum(axis=1)          # per replica
+    children = stats['cohort_offspring'].sum(axis=1)         # = agents with an infector
+    per_rep = n_agents / 8.0 + (4.0 + 32.0) * infected + 32.0 * children
+    return float(per_rep.sum()), float(infected.mean()), float(children.mean())
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument('--replicas', type=int, default=256)
+    ap.add_argument('--days', type=int, default=180)
+    ap.add_argument('--calls', type=int, default=30)
+    ap.add_argument('--out', default=None)
+    a = ap.parse_args()
+    from reina_b200 import inputs, model
+    v = inputs.default_variables()
+    args = inputs.build_context_args(v, area='HUS')
+    args['random_seed'] = 1
+    ctx = model.Context(n_replicas=a.replicas, max_days=a.days + 1, **args)
+    for iv in inputs.active_interventions(v, None):
+        ctx.add_intervention(iv)
+    ctx.run(a.days)
+    step_ms = ctx._engine.last_step_ms()
+    stats = ctx.transmission_stats()                          # warm-up: module load, table allocation
+    times = []
+    for _ in range(a.calls):
+        t0 = time.perf_counter()
+        s = ctx.transmission_stats()
+        times.append(1e3 * (time.perf_counter() - t0))
+    assert all(np.array_equal(s[k], stats[k]) for k in stats), 'repeated calls differ'
+    ms = float(np.median(times))
+    total, mean_inf, mean_child = byte_model(stats, ctx.n_agents)
+    out = dict(what='Context.transmission_stats() after a %d-day HUS run, %d replicas' % (a.days, a.replicas),
+               card=card(), calls=a.calls, ms_per_call_median=ms, ms_per_call_min=float(min(times)),
+               ms_per_call_max=float(max(times)), run_ms=step_ms, share_of_run=ms / step_ms if step_ms > 0 else None,
+               model_bytes=total, model_gbs=total / (ms / 1e3) / 1e9, hbm_gbs=HBM_GBS,
+               share_of_hbm=total / (ms / 1e3) / 1e9 / HBM_GBS, mean_infected_per_replica=mean_inf,
+               mean_children_per_replica=mean_child, agents=ctx.n_agents)
+    line = json.dumps(out)
+    print(line, flush=True)
+    if a.out:
+        with open(a.out, 'w') as f:
+            f.write(line + '\n')
+
+
+if __name__ == '__main__':
+    main()
