@@ -208,6 +208,28 @@ int rb_transmission_stats(rb_engine *e, int32_t *out);
 /* Infection day of every agent of one replica (-1 = never infected): with rb_read_agents' infector, the transmission tree. */
 int rb_read_infection_days(rb_engine *e, int32_t replica, int32_t *out);
 
+/* Transmission by setting and age of the state after the last completed rb_step (no reference counterpart: main.pyx
+ * only counts daily_contacts[place], contacts made rather than infections).  The place of a child's infection is
+ * recomputed from its infector, infection day and winning contact slot, which every run keeps, against the contact
+ * table of the epoch in force on that day.  Per replica one int32 row of rb_transmission_settings_len entries,
+ * M = max_days + 1, P = RB_N_PLACES, G = n_groups:
+ *   by_day_place[M][P + 1]     infected agents by infection day and place of infection (column RB_PLACE_ROOT: imports and
+ *                              the initial state, which have no infector)
+ *   pair_all[P][G][G]          children by place, infector's age group, child's age group
+ *   pair_closed[P][G][G]       the same, only children of closed infectors (neither INCUBATION nor ILLNESS)
+ *   closed_by_group[G]         closed cases by age group (equals group_closed of rb_transmission_stats)
+ * epoch_of_day[0 .. n_days): the contact-table epoch (rb_set_contact_table) in force on each completed day, as the caller
+ * scheduled it (rb_day_params.table_epoch); n_days must equal rb_day(e) and every epoch must have a table, else 1.
+ * Identical on every rank of a population-sharded simulation.  CUDA library only: the tests' CPU reference is the
+ * oracle, which records the place where it infects, plus these three entry points as plain loops
+ * (tests/oracle_settings.c). */
+#define RB_PLACE_ROOT RB_N_PLACES
+int32_t rb_transmission_settings_len(rb_engine *e);   /* (max_days + 1)(RB_N_PLACES + 1) + 2 RB_N_PLACES n_groups^2 + n_groups */
+/* out[n_replicas][rb_transmission_settings_len] */
+int rb_transmission_settings(rb_engine *e, const int32_t *epoch_of_day, int32_t n_days, int32_t *out);
+/* Place of infection of every agent of one replica: -1 never infected, 0 .. RB_N_PLACES - 1, RB_PLACE_ROOT. */
+int rb_read_infection_places(rb_engine *e, int32_t replica, const int32_t *epoch_of_day, int32_t n_days, int32_t *out);
+
 /* Parity/debug exports. */
 int rb_read_agents(rb_engine *e, int32_t replica, rb_agent *out);
 int rb_read_queue(rb_engine *e, int32_t replica, int32_t *out, int32_t cap, int32_t *n);   /* test queue, in order */

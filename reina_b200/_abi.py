@@ -20,6 +20,7 @@ RB_N_PLACES = 6
 RB_IOT_LEN = 21
 RB_N_TABLES = 6
 RB_TX_BINS = 65      # offspring / generation-interval histograms: bins 0..63 and ">= 64"
+RB_PLACE_ROOT = RB_N_PLACES   # place index of imports and the initial state (no infector)
 
 ATTRS = ['susceptible', 'vaccinated', 'infected', 'all_infected', 'detected', 'all_detected',
          'in_icu', 'cum_icu', 'in_ward', 'dead', 'recovered', 'non_hospital_deaths', 'new_infections']
@@ -90,13 +91,15 @@ SYMBOLS = ['create', 'destroy', 'reset', 'set_initial_state', 'step_profiled', '
 
 # transmission statistics from the infection tree; their CPU reference is test code (tests/oracle_transmission.c)
 TX_SYMBOLS = ['transmission_len', 'transmission_stats', 'read_infection_days']
+# the same tree by place of infection and age group; CPU reference: tests/oracle_settings.c (which includes the above)
+SX_SYMBOLS = ['transmission_settings_len', 'transmission_settings', 'read_infection_places']
 # exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS + SX_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -192,6 +195,7 @@ class Library:
         self.f = f
         if prefix == 'rb_':
             self.bind_transmission()
+            self.bind_settings()
 
     def bind_transmission(self):
         """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
@@ -203,6 +207,16 @@ class Library:
         f['transmission_len'].restype = C.c_int32
         f['transmission_stats'].argtypes = [vp, C.POINTER(C.c_int32)]
         f['read_infection_days'].argtypes = [vp, C.c_int32, C.POINTER(C.c_int32)]
+
+    def bind_settings(self):
+        """Bind the entry points of the tables by place of infection and age group (like bind_transmission)."""
+        f, vp = self.f, C.c_void_p
+        for name in SX_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['transmission_settings_len'].argtypes = [vp]
+        f['transmission_settings_len'].restype = C.c_int32
+        f['transmission_settings'].argtypes = [vp, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32)]
+        f['read_infection_places'].argtypes = [vp, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -405,6 +419,23 @@ class Engine:
         """Infection day of every agent of one replica, -1 = never infected."""
         out = np.empty(self.n_agents, dtype=np.int32)
         self.lib.check(self.lib.f['read_infection_days'](self.h, replica, _ptr(out, C.c_int32)), 'read_infection_days')
+        return out
+
+    def transmission_settings(self, epoch_of_day):
+        """[replica, rb_transmission_settings_len] int32: the tables by place of infection and age group of every replica
+        (reina_b200.h); epoch_of_day = contact-table epoch of every completed day."""
+        ep = np.ascontiguousarray(epoch_of_day, dtype=np.int32)
+        out = np.empty((self.n_replicas, self.lib.f['transmission_settings_len'](self.h)), dtype=np.int32)
+        self.lib.check(self.lib.f['transmission_settings'](self.h, _ptr(ep, C.c_int32), ep.size, _ptr(out, C.c_int32)),
+                       'transmission_settings')
+        return out
+
+    def read_infection_places(self, replica, epoch_of_day):
+        """Place of infection of every agent of one replica: -1 never infected, 0..5 a contact place, 6 a root."""
+        ep = np.ascontiguousarray(epoch_of_day, dtype=np.int32)
+        out = np.empty(self.n_agents, dtype=np.int32)
+        self.lib.check(self.lib.f['read_infection_places'](self.h, replica, _ptr(ep, C.c_int32), ep.size, _ptr(out, C.c_int32)),
+                       'read_infection_places')
         return out
 
     def last_step_ms(self):

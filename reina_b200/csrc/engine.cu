@@ -16,7 +16,8 @@
 //   shard.cuh     population-sharded mode: k_publish / k_wait (per-day flags in NVLink peer memory) and k_merge, which
 //                 pulls and applies every rank's message of the day
 //   setup.cuh     set_initial_state, initialisation, contact-row guide, snapshot, ensemble moments, samplers
-//   transmission.cuh  k_transmission: cohort / offspring / generation-interval tables from the infection tree (not per day)
+//   transmission.cuh  k_transmission: cohort / offspring / generation-interval tables from the infection tree (not per day);
+//                 k_transmission_settings: the same tree by place of infection and age group
 //   this file     host side: engine handle, launch geometry, replica groups, CUDA graphs, NCCL binding (ensemble reduce,
 //                 sharded mode), the extern "C" entry points
 //
@@ -89,6 +90,7 @@ struct rb_engine {
     cudaGraphExec_t sh_graph[2]; bool have_sh_graphs;      // population-sharded days (peer-memory exchange): 16 days / 1 day
     Ipc ipc; bool has_ipc;              // initial population condition, re-applied by rb_reset
     int32_t *d_tx;                      // [R][rb_transmission_len] tables of rb_transmission_stats, allocated by its first call
+    int32_t *d_sx, *d_sx_epoch;         // [R][rb_transmission_settings_len] tables, [max_days + 1] epoch of each day: allocated by the first settings call
 };
 
 // ---------------------------------------------------------------- NCCL, bound at run time
@@ -203,7 +205,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     rb_engine *e = new rb_engine();
     e->cfg = *cfg; e->day = 0; e->last_ms = 0; e->launches = 0; e->h2d_bytes = 0; e->d2h_bytes = 0; e->have_graphs = false; e->comm = nullptr; e->comm_rank = 0; e->comm_size = 1; e->sharded = false; e->merge_blocks = 1;
     e->has_ipc = false; e->h_stage = nullptr; e->n_stage = 0; e->n_groups = 1; e->wide_ctas = 1; e->n_peer_open = 0; e->launch_err = cudaSuccess; e->shard_timing = getenv("RB_SHARD_TIMING") != nullptr;
-    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr;
+    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr;
     { int lo = 0, hi = 0; CK(cudaDeviceGetStreamPriorityRange(&lo, &hi)); e->prio_high = hi; e->prio = (cfg->n_replicas >= 32 && cfg->n_replicas < 128) ? 1 : 0; if (const char *s = getenv("RB_PRIO")) e->prio = atoi(s); }
     CK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&e->ev0)); CK(cudaEventCreate(&e->ev1));
@@ -1273,6 +1275,65 @@ extern "C" int rb_read_infection_days(rb_engine *e, int32_t replica, int32_t *ou
     int32_t *d; CK(cudaMallocAsync(&d, sizeof(int32_t) * G.N, e->stream));
     k_infection_days<<<(G.N + 255) / 256, 256, 0, e->stream>>>(G, replica, d);
     e->launches += 2;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, d, sizeof(int32_t) * G.N, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaFreeAsync(d, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->d2h_bytes += (int64_t)sizeof(int32_t) * G.N;
+    return 0;
+}
+
+extern "C" int32_t rb_transmission_settings_len(rb_engine *e) { return sx_layout(e->cfg.max_days, e->cfg.n_groups).len; }
+
+// The epochs of the completed days come from the caller: after rb_load_state into a fresh engine the device schedule of
+// the past days was never uploaded, while the caller replays its plan.  Checked against the tables that have been set,
+// then copied to d_sx_epoch, after the flush of the active lists that every read of the tree starts with.
+static int settings_prologue(rb_engine *e, const int32_t *epoch_of_day, int32_t n_days) {
+    if (n_days != e->day) { snprintf(g_err, sizeof g_err, "transmission settings: %d epochs given, %d days completed", n_days, e->day); return 1; }
+    for (int d = 0; d < n_days; d++) {
+        const int ep = epoch_of_day[d];
+        if (ep < 0 || ep >= e->n_table_slots || !e->tables[ep]) { snprintf(g_err, sizeof g_err, "transmission settings: day %d: contact table %d not set", d, ep); return 1; }
+    }
+    if (!e->d_sx_epoch && dalloc(e, &e->d_sx_epoch, (size_t)e->cfg.max_days + 1)) return 1;
+    if (n_days > 0) CK(cudaMemcpyAsync(e->d_sx_epoch, epoch_of_day, sizeof(int32_t) * n_days, cudaMemcpyHostToDevice, e->stream));
+    e->h2d_bytes += (int64_t)sizeof(int32_t) * n_days;
+    k_flush_lists<<<dim3(e->sweep_blocks, e->G.R), 256, 0, e->stream>>>(e->G);
+    e->launches++;
+    return 0;
+}
+
+extern "C" int rb_transmission_settings(rb_engine *e, const int32_t *epoch_of_day, int32_t n_days, int32_t *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    const Eng &G = e->G;
+    const SxLayout L = sx_layout(G.max_days, G.n_groups);
+    const size_t bytes = sizeof(int32_t) * (size_t)G.R * L.len, smem = sizeof(int32_t) * (size_t)L.len;
+    // shared counts of one replica: 29 kB at 600 days and 16 groups; beyond 48 kB only with the opt-in
+    int smem_max = 0; CK(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, e->cfg.device));
+    if (smem > (size_t)smem_max) { snprintf(g_err, sizeof g_err, "transmission settings: %zu bytes of tables per replica exceed %d bytes of shared memory (max_days too large)", smem, smem_max); return 1; }
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(k_transmission_settings, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (!e->d_sx && dalloc(e, &e->d_sx, (size_t)G.R * L.len)) return 1;
+    if (settings_prologue(e, epoch_of_day, n_days)) return 1;
+    CK(cudaMemsetAsync(e->d_sx, 0, bytes, e->stream));
+    int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+    // the geometry of k_transmission: about two waves of 256-thread CTAs over all replicas, and no CTA without agents
+    const int per_rep = std::max(1, std::min((2 * sms * (2048 / TX_THREADS) + G.R - 1) / G.R, (G.N + TX_THREADS - 1) / TX_THREADS));
+    k_transmission_settings<<<dim3(per_rep, G.R), TX_THREADS, smem, e->stream>>>(G, L, e->d_sx_epoch, e->d_sx);
+    e->launches++;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(out, e->d_sx, bytes, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->d2h_bytes += (int64_t)bytes;
+    return 0;
+}
+
+extern "C" int rb_read_infection_places(rb_engine *e, int32_t replica, const int32_t *epoch_of_day, int32_t n_days, int32_t *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    const Eng &G = e->G;
+    if (replica < 0 || replica >= G.R) { snprintf(g_err, sizeof g_err, "bad replica"); return 1; }
+    if (settings_prologue(e, epoch_of_day, n_days)) return 1;
+    int32_t *d; CK(cudaMallocAsync(&d, sizeof(int32_t) * G.N, e->stream));
+    k_infection_places<<<(G.N + 255) / 256, 256, 0, e->stream>>>(G, replica, e->d_sx_epoch, d);
+    e->launches++;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, d, sizeof(int32_t) * G.N, cudaMemcpyDeviceToHost, e->stream));
     CK(cudaFreeAsync(d, e->stream));

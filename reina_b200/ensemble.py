@@ -132,3 +132,65 @@ def transmission_summary(stats, comm=None):
                 cohort_R_se=se, complete=out['open'] == 0, offspring_mean=m, offspring_var=v, dispersion_k=disp,
                 gi_pmf=pmf, gi_mean=float((np.arange(pmf.size) * pmf).sum()), R_by_group=r_group, R_by_variant=r_var,
                 **{name: out[name] for name in _TX_SUMS})
+
+
+def _spectral_radius(m):
+    return float(np.abs(np.linalg.eigvals(m)).max()) if m.size else np.nan
+
+
+def setting_summary(settings, comm=None):
+    """Ensemble transmission by setting and age from Context.transmission_settings() of every rank (one allreduce, like
+    transmission_summary).  With K the total number of replicas, x_r[p] the infections at place p (p < 6) in replica r
+    and c_r = sum_p x_r[p] its children (agents with an infector):
+
+      share[p]                 sum x[p] / sum c, the share of infections that happened at place p (Context.PLACE_NAMES)
+      share_se[p]              its between-replica standard error by the delta method,
+                               SE^2 = sum_r (x_r[p] - share[p] c_r)^2 / (cbar^2 K (K - 1)), cbar = sum c / K
+      incidence_by_place_mean[d, p], incidence_by_place_std[d, p]   infections per day and place (p = 6: imports and
+                               the initial state) over the replicas
+      waifw[i, j]              infections of age group j by age group i, all places and replicas (who acquires
+                               infection from whom)
+      ngm[i, j]                the empirical next-generation matrix: infections in group i per closed case of group j,
+                               sum_p pair_closed[p, j, i] / closed_by_group[j] (NaN where a group has no closed case);
+                               ngm_by_place[p] the same for the infections at place p, so ngm = sum_p ngm_by_place[p]
+      R_by_place[p]            sum pair_closed[p] / sum closed_by_group: offspring per closed case at place p
+      rho                      the spectral radius of ngm (NaN columns taken as 0)
+      rho_without[p]           the spectral radius of ngm - ngm_by_place[p]
+
+    rho_without is a first-order decomposition: it removes place p's transmissions from the matrix observed in this run
+    and holds everything else fixed -- the depletion of susceptibles, who was infected when, and behaviour.  It is not a
+    simulated counterfactual; an intervention that closes a place is evaluated by running it.
+    Also returned: the summed tables by_day_place, pair_all, pair_closed, closed_by_group, and K."""
+    comm = comm or LocalComm()
+    P = len(np.asarray(settings['pair_all'])[0])
+    bdp = np.asarray(settings['by_day_place'], dtype=np.float64)
+    x = bdp[:, :, :P].sum(axis=1)                       # [K_rank, P]
+    c = x.sum(axis=1)
+    parts = [x.sum(0), (x * x).sum(0), (x * c[:, None]).sum(0), [(c * c).sum()], bdp.sum(0), (bdp * bdp).sum(0)]
+    parts += [np.asarray(settings[k], dtype=np.float64).sum(0) for k in ('pair_all', 'pair_closed', 'closed_by_group')]
+    flat = np.concatenate([np.ravel(p) for p in parts] + [[float(bdp.shape[0])]])
+    if comm.size > 1:
+        flat = comm.allreduce(flat, 'sum')
+    out, k = [], 0
+    for p in parts:
+        n = np.size(p)
+        out.append(flat[k:k + n].reshape(np.shape(p)))
+        k += n
+    sx, sx2, sxc, (sc2,), s_bdp, s_bdp2, pair_all, pair_closed, closed = out
+    K = int(round(flat[-1]))
+    sc = sx.sum()
+    with np.errstate(divide='ignore', invalid='ignore'):
+        share = sx / sc if sc > 0 else np.full(P, np.nan)
+        cbar = sc / K
+        ss = np.maximum(sx2 - 2.0 * share * sxc + share * share * sc2, 0.0)
+        se = np.sqrt(ss / (cbar * cbar * K * (K - 1))) if K > 1 and sc > 0 else np.full(P, np.nan)
+        inc_mean, inc_std = mean_std(s_bdp, s_bdp2, K)
+        ngm_by_place = np.where(closed[None, None, :] > 0, pair_closed.transpose(0, 2, 1) / closed[None, None, :], np.nan)
+        r_place = pair_closed.sum(axis=(1, 2)) / closed.sum() if closed.sum() > 0 else np.full(P, np.nan)
+    ngm = ngm_by_place.sum(axis=0)
+    m = np.nan_to_num(ngm)
+    m_place = np.nan_to_num(ngm_by_place)
+    return dict(n_replicas=K, share=share, share_se=se, incidence_by_place_mean=inc_mean, incidence_by_place_std=inc_std,
+                waifw=pair_all.sum(axis=0), ngm=ngm, ngm_by_place=ngm_by_place, R_by_place=r_place,
+                rho=_spectral_radius(m), rho_without=np.array([_spectral_radius(m - m_place[p]) for p in range(P)]),
+                by_day_place=s_bdp, pair_all=pair_all, pair_closed=pair_closed, closed_by_group=closed)

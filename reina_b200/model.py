@@ -242,6 +242,9 @@ def ncontact_cdf(nr_contacts_by_age):
 class Context:
     """model.Context (main.pyx:1746-2101) over the CUDA engine."""
 
+    # places of infection in transmission_settings() / infection_places(): the contact places, then the roots
+    PLACE_NAMES = [CONTACT_PLACE_TO_STR[i] for i in range(_abi.RB_N_PLACES)] + ['imported/initial']
+
     def __init__(self, population_params, healthcare_params, disease_params, start_date,
                  random_seed=4321, n_replicas=1, device=0, max_days=600, contact_capacity=0.0,
                  shard=None, _library=None):
@@ -526,6 +529,37 @@ class Context:
         age = np.searchsorted(self._age_start, agent, side='right') - 1
         return dict(agent=agent.astype(np.int64), infector=infector.astype(np.int64), day=days[agent].astype(np.int64),
                     age=age.astype(np.int64))
+
+    def _epoch_of_day(self):
+        # the contact-table epoch of every completed day, from the plan (load_state replays it; the device keeps no
+        # schedule of the days before a load)
+        return np.array([dp.table_epoch for dp in self._plan[:self.day]], dtype=np.int32)
+
+    def transmission_settings(self):
+        """Where infections happened and who infected whom, per replica, from the infection tree of the current state
+        (k_transmission_settings; all arrays int64 with a leading replica axis, places in PLACE_NAMES order):
+
+          by_day_place[r, d, p]       agents infected on day d (d = 0 .. today) at place p; p = 6 (RB_PLACE_ROOT) are
+                                      imports and the initial state
+          pair_all[r, p, i, j]        infections at place p of a person of age group j by one of age group i
+          pair_closed[r, p, i, j]     the same, only by infectors that can no longer infect (closed cases)
+          closed_by_group[r, i]       closed cases of age group i: the denominator of the next-generation matrix
+
+        ensemble.setting_summary() turns these into shares by place, the next-generation matrix and its spectral
+        radius with and without each place."""
+        t = self._engine.transmission_settings(self._epoch_of_day()).astype(np.int64)
+        R, M, P, G = self.n_replicas, self.max_days + 1, _abi.RB_N_PLACES, len(self.age_group_labels)
+        k0, k1, k2 = M * (P + 1), M * (P + 1) + P * G * G, M * (P + 1) + 2 * P * G * G
+        assert t.shape[1] == k2 + G
+        return dict(by_day_place=t[:, :k0].reshape(R, M, P + 1)[:, :self.day + 1],
+                    pair_all=t[:, k0:k1].reshape(R, P, G, G), pair_closed=t[:, k1:k2].reshape(R, P, G, G),
+                    closed_by_group=t[:, k2:])
+
+    def infection_places(self, replica=0):
+        """Place of infection (index into PLACE_NAMES) of every agent of transmission_tree(replica)['agent'], in that
+        order: 0..5 the contact's place, 6 an import or the initial state."""
+        p = self._engine.read_infection_places(replica, self._epoch_of_day())
+        return p[p >= 0].astype(np.int64)
 
     def row_layout(self):
         G = len(self.age_group_labels)
