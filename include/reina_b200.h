@@ -297,6 +297,20 @@ int32_t rb_shard_exchange(rb_engine *e);        /* 0 = not sharded, 1 = ncclAllG
 int64_t rb_state_bytes(rb_engine *e);
 int rb_save_state(rb_engine *e, void *out, int64_t capacity);
 int rb_load_state(rb_engine *e, const void *in, int64_t n_bytes);
+/* Blob version 3 appends the seed history of rb_read_seeds; a version-2 blob still loads, its history taken from the
+ * loaded seeds. */
+
+/* ---- Branching replicas (no reference counterpart: the reference runs one replica from day 0 and never copies one).
+ * Replica j continues from the current state of replica src[j], drawing with seed[j] from the next rb_step on.  The copy
+ * is the state of rb_save_state plus the replica's sweep-order keys, so a copy made with the source's own seed continues
+ * exactly as the source does.  Requires 0 <= src[j] < R and src[src[j]] == src[j] for every j (a replica that is copied
+ * from keeps its own state); identity src with the current seeds is a no-op, identity src with new seeds re-seeds the
+ * futures.  Refused (return 1, rb_last_error) for a bad or chained source and in population-sharded mode; the engine
+ * stays usable.  Waits for every stream of the engine first.  CUDA library only. */
+int rb_branch(rb_engine *e, const int32_t *src, const uint32_t *seed);
+/* out[R][max_days + 1]: the draw seed of every replica on every day (days after today: the seed in force now).  No
+ * reference counterpart. */
+int rb_read_seeds(rb_engine *e, uint32_t *out);
 
 /* Measurement aids of the CUDA library (tools/phase_run.py): flag 9 makes the day-boundary kernels record the cycles
  * they spend per phase; rb_debug_phase_cycles reads the 16 accumulated counters of one replica.  No effect on results. */

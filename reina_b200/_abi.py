@@ -93,13 +93,15 @@ SYMBOLS = ['create', 'destroy', 'reset', 'set_initial_state', 'step_profiled', '
 TX_SYMBOLS = ['transmission_len', 'transmission_stats', 'read_infection_days']
 # the same tree by place of infection and age group; CPU reference: tests/oracle_settings.c (which includes the above)
 SX_SYMBOLS = ['transmission_settings_len', 'transmission_settings', 'read_infection_places']
+# branching replicas from the current state; CPU reference: tests/oracle_branch.c (which includes the above)
+BRANCH_SYMBOLS = ['branch', 'read_seeds']
 # exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS + SX_SYMBOLS
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -196,6 +198,7 @@ class Library:
         if prefix == 'rb_':
             self.bind_transmission()
             self.bind_settings()
+            self.bind_branch()
 
     def bind_transmission(self):
         """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
@@ -217,6 +220,14 @@ class Library:
         f['transmission_settings_len'].restype = C.c_int32
         f['transmission_settings'].argtypes = [vp, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32)]
         f['read_infection_places'].argtypes = [vp, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int32)]
+
+    def bind_branch(self):
+        """Bind rb_branch / rb_read_seeds (like bind_transmission)."""
+        f, vp = self.f, C.c_void_p
+        for name in BRANCH_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['branch'].argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
+        f['read_seeds'].argtypes = [vp, C.POINTER(C.c_uint32)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -436,6 +447,19 @@ class Engine:
         out = np.empty(self.n_agents, dtype=np.int32)
         self.lib.check(self.lib.f['read_infection_places'](self.h, replica, _ptr(ep, C.c_int32), ep.size, _ptr(out, C.c_int32)),
                        'read_infection_places')
+        return out
+
+    def branch(self, src, seeds):
+        """Replica j continues from the current state of replica src[j] with seed seeds[j] (rb_branch)."""
+        s = np.ascontiguousarray(src, dtype=np.int32)
+        k = np.ascontiguousarray(seeds, dtype=np.uint32)
+        assert s.shape == k.shape == (self.n_replicas,)
+        self.lib.check(self.lib.f['branch'](self.h, _ptr(s, C.c_int32), _ptr(k, C.c_uint32)), 'branch')
+
+    def read_seeds(self):
+        """[replica, max_days + 1] uint32: the draw seed of every replica on every day (rb_read_seeds)."""
+        out = np.empty((self.n_replicas, self.cfg.max_days + 1), dtype=np.uint32)
+        self.lib.check(self.lib.f['read_seeds'](self.h, _ptr(out, C.c_uint32)), 'read_seeds')
         return out
 
     def last_step_ms(self):

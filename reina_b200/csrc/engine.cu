@@ -18,6 +18,7 @@
 //   setup.cuh     set_initial_state, initialisation, contact-row guide, snapshot, ensemble moments, samplers
 //   transmission.cuh  k_transmission: cohort / offspring / generation-interval tables from the infection tree (not per day);
 //                 k_transmission_settings: the same tree by place of infection and age group
+//   branch.cuh    k_branch_copy / k_branch_rebuild: replicas continue from another replica's current state (rb_branch)
 //   this file     host side: engine handle, launch geometry, replica groups, CUDA graphs, NCCL binding (ensemble reduce,
 //                 sharded mode), the extern "C" entry points
 //
@@ -32,6 +33,7 @@
 #include "setup.cuh"
 #include "run.cuh"
 #include "transmission.cuh"
+#include "branch.cuh"
 
 // ================================================================ host side / C-ABI
 static thread_local char g_err[512];
@@ -91,6 +93,8 @@ struct rb_engine {
     Ipc ipc; bool has_ipc;              // initial population condition, re-applied by rb_reset
     int32_t *d_tx;                      // [R][rb_transmission_len] tables of rb_transmission_stats, allocated by its first call
     int32_t *d_sx, *d_sx_epoch;         // [R][rb_transmission_settings_len] tables, [max_days + 1] epoch of each day: allocated by the first settings call
+    int32_t *d_branch;                  // [R] sources then [R] seeds of rb_branch, allocated by its first call
+    uint32_t *seed_of_day;              // [R][max_days + 1] seed history (branch.cuh)
 };
 
 // ---------------------------------------------------------------- NCCL, bound at run time
@@ -147,7 +151,8 @@ static int init_population(rb_engine *e, uint32_t seed, bool sparse) {
     else k_init<false><<<dim3(e->sweep_blocks, G.R), 256, 0, e->stream>>>(G);
     k_init_bitmaps<<<dim3(8, G.R), 256, 0, e->stream>>>(G);
     k_clear_lists<<<128, 256, 0, e->stream>>>(G);
-    e->launches += 4;
+    k_init_seeds<<<G.R, 128, 0, e->stream>>>(G, e->seed_of_day, seed, 0);
+    e->launches += 5;
     CK(cudaGetLastError());
     return 0;
 }
@@ -205,7 +210,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     rb_engine *e = new rb_engine();
     e->cfg = *cfg; e->day = 0; e->last_ms = 0; e->launches = 0; e->h2d_bytes = 0; e->d2h_bytes = 0; e->have_graphs = false; e->comm = nullptr; e->comm_rank = 0; e->comm_size = 1; e->sharded = false; e->merge_blocks = 1;
     e->has_ipc = false; e->h_stage = nullptr; e->n_stage = 0; e->n_groups = 1; e->wide_ctas = 1; e->n_peer_open = 0; e->launch_err = cudaSuccess; e->shard_timing = getenv("RB_SHARD_TIMING") != nullptr;
-    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr;
+    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr; e->d_branch = nullptr;
     { int lo = 0, hi = 0; CK(cudaDeviceGetStreamPriorityRange(&lo, &hi)); e->prio_high = hi; e->prio = (cfg->n_replicas >= 32 && cfg->n_replicas < 128) ? 1 : 0; if (const char *s = getenv("RB_PRIO")) e->prio = atoi(s); }
     CK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&e->ev0)); CK(cudaEventCreate(&e->ev1));
@@ -281,6 +286,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
         dalloc(e, &G.ev_key, (size_t)R * G.cap_events) || dalloc(e, &G.ev_agent, (size_t)R * G.cap_events) ||
         dalloc(e, &G.q_key, (size_t)R * 2 * G.cap_queue) || dalloc(e, &G.q_agent, (size_t)R * 2 * G.cap_queue) ||
         dalloc(e, &G.ctr, (size_t)R) || dalloc(e, &G.stats, (size_t)R * (cfg->max_days + 1) * G.row_len) ||
+        dalloc(e, &e->seed_of_day, (size_t)R * (cfg->max_days + 1)) ||
         dalloc(e, &e->d_sched, (size_t)cfg->max_days + 1) ||
         dalloc(e, &e->d_moments, 2 * ((size_t)cfg->max_days + 1) * G.row_len + 2)) { rb_destroy(e); return 1; }
     G.sched = e->d_sched;
@@ -1205,7 +1211,7 @@ extern "C" int rb_sample(rb_engine *e, int32_t what, int32_t age, int32_t severi
     if (what < 0 || what > 6 || age < 0 || age >= e->cfg.n_ages) { snprintf(g_err, sizeof g_err, "bad sample request"); return 1; }
     int32_t *d; CK(cudaMalloc(&d, sizeof(int32_t) * n));
     int epoch = e->h_sched[e->day > 0 ? e->day - 1 : 0].table_epoch;
-    k_sample<<<(n + 255) / 256, 256, 0, e->stream>>>(e->G, what, age, severity, n, epoch, d); e->launches++;
+    k_sample<<<(n + 255) / 256, 256, 0, e->stream>>>(e->G, e->cfg.seed, what, age, severity, n, epoch, d); e->launches++;
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(e->stream));
     CK(cudaMemcpy(out, d, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
@@ -1317,7 +1323,7 @@ extern "C" int rb_transmission_settings(rb_engine *e, const int32_t *epoch_of_da
     int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
     // the geometry of k_transmission: about two waves of 256-thread CTAs over all replicas, and no CTA without agents
     const int per_rep = std::max(1, std::min((2 * sms * (2048 / TX_THREADS) + G.R - 1) / G.R, (G.N + TX_THREADS - 1) / TX_THREADS));
-    k_transmission_settings<<<dim3(per_rep, G.R), TX_THREADS, smem, e->stream>>>(G, L, e->d_sx_epoch, e->d_sx);
+    k_transmission_settings<<<dim3(per_rep, G.R), TX_THREADS, smem, e->stream>>>(G, L, e->d_sx_epoch, e->seed_of_day, e->d_sx);
     e->launches++;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, e->d_sx, bytes, cudaMemcpyDeviceToHost, e->stream));
@@ -1332,7 +1338,7 @@ extern "C" int rb_read_infection_places(rb_engine *e, int32_t replica, const int
     if (replica < 0 || replica >= G.R) { snprintf(g_err, sizeof g_err, "bad replica"); return 1; }
     if (settings_prologue(e, epoch_of_day, n_days)) return 1;
     int32_t *d; CK(cudaMallocAsync(&d, sizeof(int32_t) * G.N, e->stream));
-    k_infection_places<<<(G.N + 255) / 256, 256, 0, e->stream>>>(G, replica, e->d_sx_epoch, d);
+    k_infection_places<<<(G.N + 255) / 256, 256, 0, e->stream>>>(G, replica, e->d_sx_epoch, e->seed_of_day, d);
     e->launches++;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(out, d, sizeof(int32_t) * G.N, cudaMemcpyDeviceToHost, e->stream));
@@ -1377,12 +1383,13 @@ static std::vector<StatePart> state_parts(rb_engine *e) {
         {G.hot, RN * sizeof(uint32_t)}, {G.rec, RN * sizeof(AgentRec)}, {G.sus, RW * sizeof(uint32_t)}, {G.det, RW * sizeof(uint32_t)},
         {G.ctr, (size_t)G.R * sizeof(RepCtr)}, {G.q_key, RQ * sizeof(unsigned long long)}, {G.q_agent, RQ * sizeof(int32_t)},
         {G.stats, (size_t)G.R * (G.max_days + 1) * G.row_len * sizeof(int32_t)},
+        {e->seed_of_day, (size_t)G.R * (G.max_days + 1) * sizeof(uint32_t)},      // since version 3: the last part
     };
 }
 static StateHeader state_header(rb_engine *e) {
     const Eng &G = e->G;
     StateHeader h; memset(&h, 0, sizeof h);
-    h.magic = STATE_MAGIC; h.version = 2; h.n_agents = G.N; h.n_replicas = G.R; h.n_ages = G.n_ages; h.row_len = G.row_len;
+    h.magic = STATE_MAGIC; h.version = 3; h.n_agents = G.N; h.n_replicas = G.R; h.n_ages = G.n_ages; h.row_len = G.row_len;
     h.max_days = G.max_days; h.day = e->day; h.sus_words = G.sus_words; h.cap_queue = G.cap_queue; h.seed = e->cfg.seed;
     h.rec_bytes = (int32_t)sizeof(AgentRec); h.ctr_bytes = (int32_t)sizeof(RepCtr);
     return h;
@@ -1409,24 +1416,80 @@ extern "C" int rb_save_state(rb_engine *e, void *out, int64_t capacity) {
     return 0;
 }
 
+// A version-2 blob (saved before the seed history existed) lacks the last part; its history is filled from the loaded
+// counters' seeds, which is what it was before any rb_branch.
 extern "C" int rb_load_state(rb_engine *e, const void *in, int64_t n_bytes) {
     CK(cudaSetDevice(e->cfg.device));
-    if (n_bytes != rb_state_bytes(e)) { snprintf(g_err, sizeof g_err, "rb_load_state: %lld bytes, this engine's state is %lld", (long long)n_bytes, (long long)rb_state_bytes(e)); return 1; }
-    StateHeader h; memcpy(&h, in, sizeof h);
-    StateHeader w = state_header(e); w.day = h.day; w.seed = h.seed;
+    std::vector<StatePart> parts = state_parts(e);
+    const int64_t v2_bytes = rb_state_bytes(e) - (int64_t)parts.back().bytes;
+    StateHeader h; memset(&h, 0, sizeof h);
+    if (n_bytes >= (int64_t)sizeof h) memcpy(&h, in, sizeof h);
+    const bool v2 = h.version == 2 && n_bytes == v2_bytes;
+    if (n_bytes != rb_state_bytes(e) && !v2) { snprintf(g_err, sizeof g_err, "rb_load_state: %lld bytes, this engine's state is %lld", (long long)n_bytes, (long long)rb_state_bytes(e)); return 1; }
+    if (v2) parts.pop_back();
+    StateHeader w = state_header(e); w.day = h.day; w.seed = h.seed; if (v2) w.version = 2;
     if (memcmp(&h, &w, sizeof h) != 0) { snprintf(g_err, sizeof g_err, "rb_load_state: the blob was saved by an engine of another shape (agents / replicas / max_days / build)"); return 1; }
     if (h.day < 0 || h.day > e->cfg.max_days) { snprintf(g_err, sizeof g_err, "rb_load_state: bad day"); return 1; }
     CK(cudaStreamSynchronize(e->stream));
     const uint8_t *o = (const uint8_t *)in + sizeof h;
-    for (const StatePart &p : state_parts(e)) { CK(cudaMemcpy(p.dev, o, p.bytes, cudaMemcpyHostToDevice)); o += p.bytes; }
+    for (const StatePart &p : parts) { CK(cudaMemcpy(p.dev, o, p.bytes, cudaMemcpyHostToDevice)); o += p.bytes; }
     // every segment counter to zero, then lists `lsel` of every replica from the packed words
     k_clear_lists<<<128, 256, 0, e->stream>>>(e->G);
     k_rebuild_lists<<<dim3(e->sweep_blocks, e->G.R), 256, 0, e->stream>>>(e->G);
     e->launches += 2;
+    if (v2) { k_init_seeds<<<e->G.R, 128, 0, e->stream>>>(e->G, e->seed_of_day, 0u, 1); e->launches++; }
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(e->stream));
     e->day = h.day; e->cfg.seed = h.seed;
     bump_xepoch(e);
     CK(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+// ---------------------------------------------------------------- branching replicas (branch.cuh)
+// Every stream that may still run a kernel of this engine: its own and those of the replica groups (a branch copies
+// across groups).
+static int sync_all_streams(rb_engine *e) {
+    CK(cudaStreamSynchronize(e->stream));
+    for (int g = 0; g < e->n_groups && e->n_groups > 1; g++) CK(cudaStreamSynchronize(e->grp[g].stream));
+    return 0;
+}
+
+extern "C" int rb_branch(rb_engine *e, const int32_t *src, const uint32_t *seed) {
+    CK(cudaSetDevice(e->cfg.device));
+    const Eng &G = e->G;
+    const int R = G.R;
+    if (e->sharded) { snprintf(g_err, sizeof g_err, "rb_branch: not available in population-sharded mode (one replica, per-agent state split over the ranks)"); return 1; }
+    int n_copy = 0;
+    for (int j = 0; j < R; j++) {
+        if (src[j] < 0 || src[j] >= R) { snprintf(g_err, sizeof g_err, "rb_branch: src[%d] = %d is not a replica (0 .. %d)", j, src[j], R - 1); return 1; }
+        if (src[src[j]] != src[j]) { snprintf(g_err, sizeof g_err, "rb_branch: src[%d] = %d is itself copied from %d (chained sources)", j, src[j], src[src[j]]); return 1; }
+        n_copy += src[j] != j;
+    }
+    if (sync_all_streams(e)) return 1;
+    if (!e->d_branch && dalloc(e, &e->d_branch, 2 * (size_t)R)) return 1;
+    CK(cudaMemcpyAsync(e->d_branch, src, sizeof(int32_t) * R, cudaMemcpyHostToDevice, e->stream));
+    CK(cudaMemcpyAsync(e->d_branch + R, seed, sizeof(uint32_t) * R, cudaMemcpyHostToDevice, e->stream));
+    e->h2d_bytes += (int64_t)8 * R;
+    const int32_t *d_src = e->d_branch; const uint32_t *d_seed = (const uint32_t *)(e->d_branch + R);
+    int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
+    // about 16 CTAs per SM over the copied replicas; the columns of replicas that keep their state exit at once
+    const int per_rep = std::max(1, std::min(1024, sms * 16 / std::max(1, n_copy)));
+    // the day counters live in the active lists: into the packed words first, so that the copies carry them
+    k_flush_lists<<<dim3(e->sweep_blocks, R), 256, 0, e->stream>>>(G);
+    k_branch_copy<<<dim3(per_rep, R), 256, 0, e->stream>>>(G, e->seed_of_day, d_src, d_seed, e->day);
+    if (n_copy) k_branch_rebuild<<<dim3(e->sweep_blocks, R), 256, 0, e->stream>>>(G, d_src);
+    e->launches += n_copy ? 3 : 2;
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+extern "C" int rb_read_seeds(rb_engine *e, uint32_t *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    if (sync_all_streams(e)) return 1;
+    const size_t bytes = sizeof(uint32_t) * (size_t)e->G.R * (e->G.max_days + 1);
+    CK(cudaMemcpy(out, e->seed_of_day, bytes, cudaMemcpyDeviceToHost));
+    e->d2h_bytes += (int64_t)bytes;
     return 0;
 }

@@ -188,9 +188,9 @@ __global__ void k_moments(Eng G, int day0, double *out_sum, double *out_sq) {
 }
 
 // Context.sample, main.pyx:2047-2101
-__global__ void k_sample(Eng G, int what, int age, int severity, int n, int epoch, int32_t *out) {
+// keyed on the engine's seed, not on replica 0's counters: rb_branch may re-seed replica 0
+__global__ void k_sample(Eng G, uint32_t seed, int what, int age, int severity, int n, int epoch, int32_t *out) {
     const rb_variant *v = &G.variants[0];
-    uint32_t seed = G.ctr[0].seed;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         uint32_t pu = PU_SAMPLE | ((uint32_t)what << 8);
         int res;

@@ -89,9 +89,11 @@ __global__ void k_infection_days(Eng G, int r, int32_t *out) {
 
 // ---------------------------------------------------------------- transmission by setting and age
 // The place of a child's infection is not stored anywhere, but it is a pure function of what is: every draw is keyed on
-// (replica seed, agent, day, purpose | slot), and the child's record holds its infector and inf_key = day << 8 | slot
-// of the contact slot that won.  Recomputing that slot's 24-bit uniform and picking the row against the contact table
-// of that day's epoch gives the row k_expose picked, hence the place.  The row is found by an upper-bound binary search
+// (replica seed in force that day, agent, day, purpose | slot), and the child's record holds its infector and
+// inf_key = day << 8 | slot of the contact slot that won.  The seed comes from the seed history seed_of_day[R][max_days + 1]
+// (branch.cuh), not from RepCtr::seed: rb_branch gives a replica a new seed, and a child infected before that was drawn
+// with the old one.  Recomputing that slot's 24-bit uniform and picking the row against the contact table of that day's
+// epoch gives the row k_expose picked, hence the place.  The row is found by an upper-bound binary search
 // over cum24 (non-decreasing, so the search returns the linear scan's first row with k24 < cum24[row]), independent of
 // the 4096-cell guide k_expose decodes.
 //
@@ -131,17 +133,17 @@ __device__ __forceinline__ int contact_place(const DevTable *tb, uint32_t seed, 
 }
 
 // The infection place of an agent that has left SUSCEPTIBLE: RB_PLACE_ROOT for a root.
-__device__ __forceinline__ int infection_place(const Eng &G, int r, const AgentRec &rec, const int32_t *epoch_of_day) {
+__device__ __forceinline__ int infection_place(const Eng &G, int r, const AgentRec &rec, const int32_t *epoch_of_day, const uint32_t *seed_of_day) {
     if (rec.infector < 0) return RB_PLACE_ROOT;
     const uint32_t d = rec.inf_key >> 8;
-    return contact_place(G.tables[__ldg(&epoch_of_day[d])], G.ctr[r].seed, rec.infector, age_of(G, rec.infector), d, rec.inf_key & 255u);
+    return contact_place(G.tables[__ldg(&epoch_of_day[d])], seed_of_day[(size_t)r * (G.max_days + 1) + d], rec.infector, age_of(G, rec.infector), d, rec.inf_key & 255u);
 }
 
 // Same skeleton as k_transmission: blockIdx.y = replica, grid-stride over the agents, the never infected skipped through
 // the susceptibility bitmap, counts in shared memory added to out[replica] with integer atomics (geometry-independent).
 // Per child one gathered packed word of the infector (its state) and one Philox block; the contact tables are read
 // through L1 / L2.
-__global__ void __launch_bounds__(TX_THREADS) k_transmission_settings(Eng G, SxLayout L, const int32_t *epoch_of_day, int32_t *out) {
+__global__ void __launch_bounds__(TX_THREADS) k_transmission_settings(Eng G, SxLayout L, const int32_t *epoch_of_day, const uint32_t *seed_of_day, int32_t *out) {
     extern __shared__ int32_t s_sx[];
     const int r = blockIdx.y;
     const size_t base = (size_t)r * G.Npad;
@@ -163,7 +165,7 @@ __global__ void __launch_bounds__(TX_THREADS) k_transmission_settings(Eng G, SxL
         if (inf >= 0) {
             const uint32_t ist = H_STATE(G.hot[base + inf]);
             const int iage = age_of(G, inf);
-            place = contact_place(G.tables[__ldg(&epoch_of_day[d])], G.ctr[r].seed, inf, iage, (uint32_t)d, key & 255u);
+            place = contact_place(G.tables[__ldg(&epoch_of_day[d])], seed_of_day[(size_t)r * (G.max_days + 1) + d], inf, iage, (uint32_t)d, key & 255u);
             const int cell = (place * NG + __ldg(&G.group_of_age[iage])) * NG + cg;
             atomicAdd(&s_sx[L.pair_all + cell], 1);
             if (ist != RB_INCUBATION && ist != RB_ILLNESS) atomicAdd(&s_sx[L.pair_closed + cell], 1);
@@ -179,10 +181,10 @@ __global__ void __launch_bounds__(TX_THREADS) k_transmission_settings(Eng G, SxL
 
 // Infection place of every agent of one replica (rb_read_infection_places): -1 never infected, 0 .. RB_N_PLACES - 1 the
 // place of the contact, RB_PLACE_ROOT an import or the initial state.
-__global__ void k_infection_places(Eng G, int r, const int32_t *epoch_of_day, int32_t *out) {
+__global__ void k_infection_places(Eng G, int r, const int32_t *epoch_of_day, const uint32_t *seed_of_day, int32_t *out) {
     const size_t base = (size_t)r * G.Npad;
     for (int a = blockIdx.x * blockDim.x + threadIdx.x; a < G.N; a += gridDim.x * blockDim.x)
-        out[a] = H_STATE(G.hot[base + a]) == RB_SUSCEPTIBLE ? -1 : infection_place(G, r, G.rec[base + a], epoch_of_day);
+        out[a] = H_STATE(G.hot[base + a]) == RB_SUSCEPTIBLE ? -1 : infection_place(G, r, G.rec[base + a], epoch_of_day, seed_of_day);
 }
 
 #endif

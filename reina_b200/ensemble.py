@@ -8,6 +8,8 @@ bands gather the members' rows over the same communicator.  Replaces the referen
 pool (calc/simulation.py:349-385).  No framework is imported here: a communicator is any object with rank / size /
 allreduce / allgather / barrier (reina_b200/comm.py; the CPU tests pass an adapter over a gloo group).
 """
+import math
+
 import numpy as np
 
 from .comm import LocalComm
@@ -194,3 +196,131 @@ def setting_summary(settings, comm=None):
                 waifw=pair_all.sum(axis=0), ngm=ngm, ngm_by_place=ngm_by_place, R_by_place=r_place,
                 rho=_spectral_radius(m), rho_without=np.array([_spectral_radius(m - m_place[p]) for p in range(P)]),
                 by_day_place=s_bdp, pair_all=pair_all, pair_closed=pair_closed, closed_by_group=closed)
+
+
+# ---------------------------------------------------------------- conditioning on observed counts
+def systematic_resample(weights, rng):
+    """Systematic resampling: how many copies of each replica to keep, counts[r] >= 0 with sum R, for normalised or
+    unnormalised weights >= 0 (one uniform from the numpy Generator `rng`)."""
+    w = np.asarray(weights, dtype=np.float64)
+    if w.ndim != 1 or w.size == 0 or not np.isfinite(w).all() or (w < 0).any() or not w.sum() > 0:
+        raise ValueError('weights must be finite, >= 0 and not all 0')
+    R = w.size
+    cum = np.cumsum(w / w.sum())
+    cum[-1] = 1.0
+    idx = np.searchsorted(cum, (rng.random() + np.arange(R)) / R, side='right')
+    return np.bincount(np.minimum(idx, R - 1), minlength=R)
+
+
+def assign_slots(counts):
+    """The `source` of Context.branch for resampling counts: a replica with counts >= 1 keeps its slot, its extra copies
+    fill the slots of the replicas with count 0 in increasing order.  So source[source[j]] == source[j] always."""
+    c = np.asarray(counts, dtype=np.int64)
+    if c.ndim != 1 or (c < 0).any() or c.sum() != c.size:
+        raise ValueError('counts must be >= 0 and sum to their number')
+    src = np.arange(c.size)
+    src[c == 0] = np.repeat(np.arange(c.size), np.maximum(c - 1, 0))
+    return src.astype(np.int32)
+
+
+def _lgamma(x):
+    return np.vectorize(math.lgamma, otypes=[np.float64])(x)
+
+
+def log_likelihood(mean, observed, model='negbin', dispersion=10.0):
+    """log P(observed | model count `mean`) per replica: negative binomial with that mean and dispersion k (variance
+    mean + mean^2 / k), or Poisson.  A mean of 0 gives 0 for an observed 0 and -inf otherwise."""
+    mu = np.asarray(mean, dtype=np.float64)
+    y = float(observed)
+    if y < 0 or y != int(y):
+        raise ValueError('an observed count must be a non-negative integer, got %r' % observed)
+    with np.errstate(divide='ignore', invalid='ignore'):
+        if model == 'poisson':
+            ll = y * np.log(mu) - mu - math.lgamma(y + 1.0)
+        elif model == 'negbin':
+            k = float(dispersion)
+            if not k > 0:
+                raise ValueError('dispersion must be > 0')
+            ll = (_lgamma(y + k) - math.lgamma(k) - math.lgamma(y + 1.0) + k * np.log(k / (k + mu))
+                  + y * np.log(mu / (k + mu)))
+        else:
+            raise ValueError("model must be 'negbin' or 'poisson'")
+    return np.where(mu > 0, ll, 0.0 if y == 0 else -np.inf)
+
+
+def _model_counts(ctx, rows, name):
+    """Column `name` of stats rows [replica, row]: an ATTRS name summed over the age groups, or a row_layout() column."""
+    from ._abi import ATTRS
+    G = len(ctx.age_group_labels)
+    if name in ATTRS:
+        i = ATTRS.index(name)
+        return rows[:, i * G:(i + 1) * G].sum(axis=1)
+    names = ctx.row_layout()
+    if name not in names:
+        raise ValueError('unknown observation %r: an ATTRS name or a row_layout() column' % name)
+    return rows[:, names.index(name)]
+
+
+def _logsumexp(x):
+    m = x.max()
+    return m + math.log(np.exp(x - m).sum()) if np.isfinite(m) else m
+
+
+def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0):
+    """Sequential importance resampling of the replicas of ONE Context against observed counts.
+
+    observations = {day: {name: count}}: `name` is an ATTRS name summed over the age groups ('in_ward', 'in_icu',
+    'dead', 'all_detected', ...) or a row_layout() column.  The observation of day d is compared with stats row d, the
+    state before the d-th iterate() (what generate_state() returns at ctx.day == d); the days must not lie before
+    ctx.day.  The likelihood of a replica is a negative binomial with mean equal to its count and dispersion k
+    (`dispersion`), or Poisson (model='poisson'); several names on one day are independent.  After each observation
+    day the weights are updated, and when the effective sample size falls below ess_threshold * R -- and always at the
+    last observation -- the replicas are resampled systematically (systematic_resample with a Generator seeded by
+    `seed`) and copied on the device with Context.branch (assign_slots): every copy continues with a fresh seed.
+
+    The Context is left at the last observation day, equally weighted, so run(), series(), moments() and
+    percentile_bands() give the forecast from there.  The rows of days before it are the paths of the surviving
+    replicas' ancestors: for early days few distinct paths remain (they degenerate), so read the past from the filter's
+    weights at each day, not from the returned ensemble.  Resampling across GPUs (moving replica state between ranks) is
+    not provided: every rank filters its own replicas.
+
+    Returns a dict: log_evidence (the sum over the observation days of the log mean incremental weight), days[k],
+    ess[k] (before resampling), resampled[k], ancestors[k, R] (the branch source of step k, the identity where nothing
+    was resampled) and loglik[k, R].  Raises ValueError naming the day if no replica can explain an observation (every
+    weight zero)."""
+    R = ctx.n_replicas
+    days = sorted(int(d) for d in observations)
+    if days and (days[0] < ctx.day or days[-1] > ctx.max_days):
+        raise ValueError('observation days must lie in [ctx.day, max_days] = [%d, %d]' % (ctx.day, ctx.max_days))
+    rng = np.random.default_rng(seed)
+    logw = np.full(R, -math.log(R))
+    out = dict(log_evidence=0.0, days=np.array(days, dtype=np.int64), ess=np.zeros(len(days)),
+               resampled=np.zeros(len(days), dtype=bool), ancestors=np.zeros((len(days), R), dtype=np.int32),
+               loglik=np.zeros((len(days), R)))
+    for k, d in enumerate(days):
+        if d > ctx.day:
+            ctx.run(d - ctx.day)
+        ctx._engine.snapshot()
+        ctx._engine.sync()
+        ctx._state_day = ctx.day
+        rows = ctx._engine.read_stats(d, 1)[:, 0].astype(np.float64)
+        ll = np.zeros(R)
+        for name, y in observations[d].items():
+            ll += log_likelihood(_model_counts(ctx, rows, name), y, model, dispersion)
+        post = logw + ll
+        total = _logsumexp(post)
+        if not np.isfinite(total):
+            raise ValueError('particle_filter: no replica can explain the observations of day %d (every weight is 0)' % d)
+        out['log_evidence'] += total                  # logw is normalised: log sum_j W_j exp(ll_j)
+        logw = post - total
+        w = np.exp(logw)
+        ess = 1.0 / (w * w).sum()
+        src = np.arange(R, dtype=np.int32)
+        if ess < ess_threshold * R or k == len(days) - 1:
+            src = assign_slots(systematic_resample(w, rng))
+            if (src != np.arange(R)).any():
+                ctx.branch(src)
+            logw = np.full(R, -math.log(R))
+            out['resampled'][k] = True
+        out['ess'][k], out['ancestors'][k], out['loglik'][k] = ess, src, ll
+    return out

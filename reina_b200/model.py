@@ -561,6 +561,41 @@ class Context:
         p = self._engine.read_infection_places(replica, self._epoch_of_day())
         return p[p >= 0].astype(np.int64)
 
+    def branch(self, source, seeds=None):
+        """Many futures of one present (rb_branch): replica j continues from the current state of replica source[j] --
+        agents, infection tree, test queue, counters and its stats rows so far -- and draws with its own seed from the
+        next iterate() on.  `source` is an int array of length n_replicas, or one int: every replica from that one.  A
+        replica that is copied from keeps its own state (source[source[j]] == source[j]).
+
+        seeds None: every replica whose state changes (source[j] != j) gets a seed this engine has never used, the others
+        keep theirs; else an array of n_replicas seeds (a copy given its source's seed continues exactly as the source).
+        Returns the seeds now in force.  Rows of days before today are the source's; today's row is written by the next
+        iterate() or generate_state()."""
+        R = self.n_replicas
+        src = np.full(R, int(source), dtype=np.int64) if np.ndim(source) == 0 else np.asarray(source, dtype=np.int64)
+        if src.shape != (R,):
+            raise ValueError('source must be one int or %d ints' % R)
+        hist = self._engine.read_seeds()
+        if seeds is None:
+            seeds = hist[:, self.day].copy()
+            used = set(hist.ravel().tolist())
+            nxt = int(hist.max()) + 1
+            for j in np.flatnonzero(src != np.arange(R)):
+                while (nxt & 0xFFFFFFFF) in used:
+                    nxt += 1
+                seeds[j] = nxt & 0xFFFFFFFF
+                used.add(int(seeds[j]))
+        seeds = np.asarray(seeds, dtype=np.int64)
+        if seeds.shape != (R,) or (seeds < 0).any() or (seeds > 0xFFFFFFFF).any():
+            raise ValueError('seeds must be %d unsigned 32-bit ints' % R)
+        self._engine.branch(src, seeds.astype(np.uint32))
+        self._state_day = -1
+        return seeds.astype(np.uint32)
+
+    def replica_seeds(self):
+        """The seed every replica draws with from today on (random_seed + r until a branch changes it)."""
+        return self._engine.read_seeds()[:, self.day].copy()
+
     def row_layout(self):
         G = len(self.age_group_labels)
         names = ['%s[%s]' % (a, g) for a in ATTRS for g in self.age_group_labels]
