@@ -8,7 +8,7 @@
 // replica is both read and written.
 //
 // The seed history seed_of_day[R][max_days + 1] (the seed of every replica on every day) is a kernel argument, not a
-// member of Eng: a larger Eng would move the parameters k_run takes after it, and the per-day kernels stay as built.
+// member of Eng: Eng is every per-day kernel's parameter block, and those kernels stay as built.
 #ifndef REINA_B200_BRANCH_CUH
 #define REINA_B200_BRANCH_CUH
 

@@ -12,7 +12,6 @@
 //                 segments); emits contact work items, capacity events and test-queue entries tagged with sweep position
 //   contacts.cuh  k_expose: one thread per group of four sampled contacts (O(1) row pick, target gather, transmission
 //                 draw, atomicMin(winner[target], sweep position of infector | slot)); k_resolve: winners become infected
-//   run.cuh       k_run: opt-in persistent cooperative kernel, the whole run of a few replicas in one launch
 //   shard.cuh     population-sharded mode: k_publish / k_wait (per-day flags in NVLink peer memory) and k_merge, which
 //                 pulls and applies every rank's message of the day
 //   setup.cuh     set_initial_state, initialisation, contact-row guide, snapshot, ensemble moments, samplers
@@ -31,7 +30,6 @@
 #include "contacts.cuh"
 #include "shard.cuh"
 #include "setup.cuh"
-#include "run.cuh"
 #include "transmission.cuh"
 #include "branch.cuh"
 
@@ -69,15 +67,13 @@ struct rb_engine {
     float last_ms;
     int64_t launches;
     int64_t h2d_bytes, d2h_bytes;       // bytes this handle copied host -> device / device -> host so far (rb_copied_bytes)
-    int sweep_blocks, list_blocks, resolve_blocks;
-    cudaGraphExec_t graph[2];
+    int sweep_blocks, list_blocks, resolve_blocks;     // full-wave grids over all replicas
     bool have_graphs;
     // replica groups: the ensemble is split into n_groups sets of replicas, each advanced by its own chain of launches
     // on its own stream with a grid sized for its share of the SMs.  The groups run half a day apart, so the
     // latency-bound phases of one (k_resolve, the single-CTA day boundary) overlap the sweep / contact kernels of another.
     cudaError_t launch_err;             // first failed cooperative launch (launch_boundary)
     int wide_ctas;                      // CTAs per replica of the wide day boundary (<= 1: one CTA per replica)
-    int run_ctas, run_boundary_ctas;    // k_run (few replicas): CTAs per replica of the persistent run kernel (0: not used), of its boundary sub-team
     int n_groups;
     ReplicaGroup grp[MAX_GROUPS];
     cudaEvent_t ev_fork;
@@ -89,7 +85,6 @@ struct rb_engine {
     int merge_blocks;
     int prio, prio_high;                // RB_PRIO: launch the latency-bound kernels with the device's highest priority
     uint32_t xepoch; uint32_t *d_xepoch;   // host copy / device word of Eng::xepoch
-    cudaGraphExec_t sh_graph[2]; bool have_sh_graphs;      // population-sharded days (peer-memory exchange): 16 days / 1 day
     Ipc ipc; bool has_ipc;              // initial population condition, re-applied by rb_reset
     int32_t *d_tx;                      // [R][rb_transmission_len] tables of rb_transmission_stats, allocated by its first call
     int32_t *d_sx, *d_sx_epoch;         // [R][rb_transmission_settings_len] tables, [max_days + 1] epoch of each day: allocated by the first settings call
@@ -176,15 +171,11 @@ extern "C" void rb_destroy(rb_engine *e) {
     if (!e) return;
     cudaSetDevice(e->cfg.device);
     cudaStreamSynchronize(e->stream);
-    if (e->have_graphs) {
-        if (e->n_groups <= 1) { cudaGraphExecDestroy(e->graph[0]); cudaGraphExecDestroy(e->graph[1]); }
-        else for (int g = 0; g < e->n_groups; g++) { cudaGraphExecDestroy(e->grp[g].graph[0]); cudaGraphExecDestroy(e->grp[g].graph[1]); }
-    }
+    if (e->have_graphs) for (int g = 0; g < e->n_groups; g++) { cudaGraphExecDestroy(e->grp[g].graph[0]); cudaGraphExecDestroy(e->grp[g].graph[1]); }
     for (int g = 0; g < e->n_groups && e->n_groups > 1; g++) {
         cudaStreamDestroy(e->grp[g].stream); cudaEventDestroy(e->grp[g].ev_stagger); cudaEventDestroy(e->grp[g].ev_join);
     }
     if (e->n_groups > 1) cudaEventDestroy(e->ev_fork);
-    if (e->have_sh_graphs) { cudaGraphExecDestroy(e->sh_graph[0]); cudaGraphExecDestroy(e->sh_graph[1]); }
     for (int k = 0; k < e->n_peer_open; k++) if (k != e->G.rank && e->G.xpeer[k]) cudaIpcCloseMemHandle(e->G.xpeer[k]);
     if (e->comm) g_nccl.CommDestroy(e->comm);
     for (void *p : e->allocs) cudaFree(p);
@@ -210,7 +201,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     rb_engine *e = new rb_engine();
     e->cfg = *cfg; e->day = 0; e->last_ms = 0; e->launches = 0; e->h2d_bytes = 0; e->d2h_bytes = 0; e->have_graphs = false; e->comm = nullptr; e->comm_rank = 0; e->comm_size = 1; e->sharded = false; e->merge_blocks = 1;
     e->has_ipc = false; e->h_stage = nullptr; e->n_stage = 0; e->n_groups = 1; e->wide_ctas = 1; e->n_peer_open = 0; e->launch_err = cudaSuccess; e->shard_timing = getenv("RB_SHARD_TIMING") != nullptr;
-    e->xepoch = 0; e->d_xepoch = nullptr; e->have_sh_graphs = false; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr; e->d_branch = nullptr;
+    e->xepoch = 0; e->d_xepoch = nullptr; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr; e->d_branch = nullptr;
     { int lo = 0, hi = 0; CK(cudaDeviceGetStreamPriorityRange(&lo, &hi)); e->prio_high = hi; e->prio = (cfg->n_replicas >= 32 && cfg->n_replicas < 128) ? 1 : 0; if (const char *s = getenv("RB_PRIO")) e->prio = atoi(s); }
     CK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&e->ev0)); CK(cudaEventCreate(&e->ev1));
@@ -244,27 +235,6 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     const size_t RN = (size_t)R * G.Npad;
     cudaDeviceProp prop; CK(cudaGetDeviceProperties(&prop, cfg->device));
     const int sms = prop.multiProcessorCount;
-    // Few replicas: the whole run as one persistent cooperative kernel, a team of co-resident CTAs per replica (run.cuh):
-    // ONE launch per rb_step instead of four per day.  Opt-in (RB_PERSISTENT=1, team size RB_RUN_CTAS): measured on B200 it
-    // does not beat the graph-replayed kernels -- one HUS replica 58.0 us per day with a team of 148 CTAs (62.2 with 64,
-    // 78.6 with 16) against 55.1, 32 replicas 24.4 ms per run against 22.8 -- because a day of few replicas is bound by the
-    // dependent memory round trips INSIDE its phases (lead CTA of one replica: sweep 6.3 + 5.9 us waiting for the slowest
-    // warp, contacts 8.4, resolve 10.7, day boundary 27.6), not by the launches between them.
-    e->run_ctas = 0; e->run_boundary_ctas = 1;
-    {
-        int per_sm = 0;
-        CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_run, RUN_THREADS, 0));
-        const long long total = (long long)per_sm * sms;
-        bool on = false;
-        if (const char *s = getenv("RB_PERSISTENT")) on = atoi(s) != 0;
-        if (on && total >= 2LL * R) {
-            long long t = total / R; if (t > 64) t = 64;
-            if (const char *s = getenv("RB_RUN_CTAS")) { const int v = atoi(s); if (v >= 1 && (long long)v * R <= total) t = v; }
-            e->run_ctas = (int)t;
-            int b = 1; while (b * 2 <= t && b * 2 <= 16) b *= 2;        // the boundary's team sort wants a power of two
-            e->run_boundary_ctas = b;
-        }
-    }
     {   // Active-list segments (state.cuh, Eng::alist)
         // two per warp of the sweep grid a replica gets in the production geometry (its replica group's share of a wave):
         // a warp streams a segment from end to end, so segments are the unit of load balance -- but every segment costs a
@@ -275,7 +245,6 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
         long long ctas = (long long)sms * SW_CTAS_PER_SM * (ng > 1 ? pct : 100) / 100 / ((R + ng - 1) / ng);      // as setup_groups sizes the grid
         if (ctas < 1) ctas = 1;
         long long S = 2 * ctas * SW_WARPS, most = (long long)N / 256;
-        if (e->run_ctas) S = 2LL * e->run_ctas * RUN_WARPS;
         if (S > most) S = most;
         G.n_seg = (uint32_t)(S < 1 ? 1 : S);
         G.seg_cap = ((uint32_t)N + G.n_seg - 1) / G.n_seg;        // agents a with a % n_seg == s: never more than this
@@ -333,8 +302,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     e->resolve_blocks = resolve_grid(G.N, sms, 100, R);
     if (init_population(e, cfg->seed, false)) { rb_destroy(e); return 1; }
     CK(cudaStreamSynchronize(e->stream));
-    if (e->run_ctas) e->n_groups = 1;
-    else if (setup_groups(e, sms)) { rb_destroy(e); return 1; }
+    if (setup_groups(e, sms)) { rb_destroy(e); return 1; }
     // wide day boundary: only without replica groups (two wide launches on concurrent streams could each hold half
     // the SMs and wait for the other), one CTA per SM at most
     e->wide_ctas = 1;
@@ -346,10 +314,6 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     if (e->n_groups == 1 && R * 4 <= sms && N >= 4000000) { e->wide_ctas = 16; while (e->wide_ctas * R > sms) e->wide_ctas >>= 1; }     // a power of two (team sort)
     if (const char *s = getenv("RB_WIDE_CTAS")) { int v = atoi(s); if (v >= 1 && v <= WIDE_MAX_CTAS && v * R <= sms) e->wide_ctas = v; }
     if (const char *s = getenv("RB_WIDE_MIN")) G.wide_min = atoi(s);     // 0: every day is a wide day (tests)
-    if (const char *s = getenv("RB_WIDE_CTAS")) {      // tests force a boundary team of this size in the persistent kernel too
-        const int v = atoi(s); int b = 1; while (b * 2 <= v && b * 2 <= e->run_ctas) b *= 2;
-        if (e->run_ctas) e->run_boundary_ctas = b;
-    }
     *out = e;
     return 0;
 }
@@ -376,7 +340,12 @@ static int setup_groups(rb_engine *e, int sms) {
     int ng, pct;
     group_config(R, &ng, &pct);
     e->n_groups = ng;
-    if (ng == 1) return 0;
+    if (ng == 1) {      // the whole ensemble on the engine's own stream with the full-wave grids, whatever `pct` says
+        ReplicaGroup &q = e->grp[0];
+        q.r0 = 0; q.R = R; q.sweep_blocks = e->sweep_blocks; q.list_blocks = e->list_blocks; q.resolve_blocks = e->resolve_blocks;
+        q.stream = e->stream;
+        return 0;
+    }
     CK(cudaEventCreateWithFlags(&e->ev_fork, cudaEventDisableTiming));
     const Eng &G = e->G;
     const int want = ((int)G.n_seg + SW_WARPS - 1) / SW_WARPS;
@@ -586,15 +555,7 @@ static void launch_boundary(rb_engine *e, int kind, int R, cudaStream_t st, cons
     if (err != cudaSuccess && e->launch_err == cudaSuccess) e->launch_err = err;     // reported by the rb_step that issued it
 }
 
-// One "segment" = the grid kernels of day d followed by the fused day boundary d -> d+1.
-static void launch_segment(rb_engine *e, cudaStream_t st) {
-    const Eng &G = e->G;
-    launch_k(e, k_sweep, dim3(e->sweep_blocks, G.R), SW_THREADS, st, G);
-    launch_k(e, k_expose, dim3(e->list_blocks, G.R), EX_THREADS, st, G);
-    launch_k(e, k_resolve<true>, dim3(e->resolve_blocks, G.R), 256, st, G, true);
-    launch_boundary(e, 2, G.R, st, G);
-}
-
+// One "segment" = the grid kernels of day d followed by the fused day boundary d -> d+1, for one replica group.
 // No kernel takes the day as an argument (each replica carries its own day counter and reads the schedule from
 // device memory), so a captured graph of GRAPH_DAYS segments is replayed for any stretch of days.
 static void launch_group_segment(rb_engine *e, const ReplicaGroup &q, bool stagger_mark) {
@@ -608,30 +569,17 @@ static void launch_group_segment(rb_engine *e, const ReplicaGroup &q, bool stagg
 
 #define GRAPH_DAYS 16
 static int build_graphs(rb_engine *e) {
-    if (e->n_groups > 1) {
-        for (int g = 0; g < e->n_groups; g++)
-            for (int which = 0; which < 2; which++) {
-                ReplicaGroup &q = e->grp[g];
-                int nseg = which == 0 ? GRAPH_DAYS : 1;
-                cudaGraph_t gr;
-                CK(cudaStreamBeginCapture(q.stream, cudaStreamCaptureModeThreadLocal));
-                for (int i = 0; i < nseg; i++) launch_group_segment(e, q, false);
-                CK(cudaStreamEndCapture(q.stream, &gr));
-                CK(cudaGraphInstantiate(&q.graph[which], gr, e->prio ? cudaGraphInstantiateFlagUseNodePriority : 0));
-                CK(cudaGraphDestroy(gr));
-            }
-        e->have_graphs = true;
-        return 0;
-    }
-    for (int which = 0; which < 2; which++) {
-        int nseg = which == 0 ? GRAPH_DAYS : 1;
-        cudaGraph_t g;
-        CK(cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal));
-        for (int i = 0; i < nseg; i++) launch_segment(e, e->stream);
-        CK(cudaStreamEndCapture(e->stream, &g));
-        CK(cudaGraphInstantiate(&e->graph[which], g, e->prio ? cudaGraphInstantiateFlagUseNodePriority : 0));
-        CK(cudaGraphDestroy(g));
-    }
+    for (int g = 0; g < e->n_groups; g++)
+        for (int which = 0; which < 2; which++) {
+            ReplicaGroup &q = e->grp[g];
+            int nseg = which == 0 ? GRAPH_DAYS : 1;
+            cudaGraph_t gr;
+            CK(cudaStreamBeginCapture(q.stream, cudaStreamCaptureModeThreadLocal));
+            for (int i = 0; i < nseg; i++) launch_group_segment(e, q, false);
+            CK(cudaStreamEndCapture(q.stream, &gr));
+            CK(cudaGraphInstantiate(&q.graph[which], gr, e->prio ? cudaGraphInstantiateFlagUseNodePriority : 0));
+            CK(cudaGraphDestroy(gr));
+        }
     e->have_graphs = true;
     return 0;
 }
@@ -708,7 +656,8 @@ extern "C" int rb_shard_unique_id(uint8_t *out128) {
 static int shard_prepare(rb_engine *e, int32_t rank, int32_t nranks, float exchange_capacity) {
     if (nranks < 1 || nranks > MAX_RANKS || rank < 0 || rank >= nranks) { snprintf(g_err, sizeof g_err, "bad rank %d / %d", rank, nranks); return 1; }
     if (e->G.R != 1) { snprintf(g_err, sizeof g_err, "population-sharded mode runs one replica (n_replicas = %d)", e->G.R); return 1; }
-    if (e->day != 0 || e->comm || e->sharded) { snprintf(g_err, sizeof g_err, "rb_shard_init must be the first call after rb_create"); return 1; }
+    // (have_graphs: stepped and reset -- grp[0].graph would hold unsharded days, build_shard_graphs puts sharded ones there)
+    if (e->day != 0 || e->have_graphs || e->comm || e->sharded) { snprintf(g_err, sizeof g_err, "rb_shard_init must be the first call after rb_create"); return 1; }
     CK(cudaSetDevice(e->cfg.device));
     Eng &G = e->G;
     // message capacities: this rank's share of the agents; a day's state changes / transmissions / tests / capacity
@@ -882,7 +831,8 @@ static int launch_day_sharded(rb_engine *e, bool last) {
 
 // Sharded days with the peer-memory exchange are pure kernel chains (the flag wait is a kernel too) that take no
 // per-day argument -- the day and the flag epoch are read from device memory -- so they are captured once, as graphs of
-// GRAPH_DAYS days and of one day, and replayed like the single-GPU segments.
+// GRAPH_DAYS days and of one day, and replayed like the single-GPU segments.  They are kept as the graphs of the one
+// replica group a sharded engine has (one replica): its unsharded graphs are never built.
 static int build_shard_graphs(rb_engine *e) {
     for (int which = 0; which < 2; which++) {
         const int nseg = which == 0 ? GRAPH_DAYS : 1;
@@ -890,10 +840,10 @@ static int build_shard_graphs(rb_engine *e) {
         CK(cudaStreamBeginCapture(e->stream, cudaStreamCaptureModeThreadLocal));
         for (int i = 0; i < nseg; i++) if (launch_day_sharded(e, false)) { cudaStreamEndCapture(e->stream, &g); return 1; }
         CK(cudaStreamEndCapture(e->stream, &g));
-        CK(cudaGraphInstantiate(&e->sh_graph[which], g, 0));
+        CK(cudaGraphInstantiate(&e->grp[0].graph[which], g, 0));
         CK(cudaGraphDestroy(g));
     }
-    e->have_sh_graphs = true;
+    e->have_graphs = true;
     return 0;
 }
 
@@ -921,18 +871,18 @@ extern "C" int rb_step(rb_engine *e, int32_t n_days) {
     CK(cudaSetDevice(e->cfg.device));
     if (check_days(e, n_days)) return 1;
     if (n_days == 0) return 0;
-    if (!e->sharded && !e->run_ctas && !e->have_graphs && build_graphs(e)) return 1;
+    if (!e->sharded && !e->have_graphs && build_graphs(e)) return 1;
     const Eng &G = e->G;
     const int R = G.R;
     if (e->sharded) {
         const bool graphs = G.xp2p && !e->shard_timing;
-        if (graphs && !e->have_sh_graphs && build_shard_graphs(e)) return 1;
+        if (graphs && !e->have_graphs && build_shard_graphs(e)) return 1;
         CK(cudaEventRecord(e->ev0, e->stream));
         launch_boundary(e, 0, 1, e->stream, G); e->launches++;
         int mid = n_days - 1;
         if (graphs) {
-            while (mid >= GRAPH_DAYS) { CK(cudaGraphLaunch(e->sh_graph[0], e->stream)); mid -= GRAPH_DAYS; }
-            while (mid > 0) { CK(cudaGraphLaunch(e->sh_graph[1], e->stream)); mid -= 1; }
+            while (mid >= GRAPH_DAYS) { CK(cudaGraphLaunch(e->grp[0].graph[0], e->stream)); mid -= GRAPH_DAYS; }
+            while (mid > 0) { CK(cudaGraphLaunch(e->grp[0].graph[1], e->stream)); mid -= 1; }
         } else for (; mid > 0; mid--) if (launch_day_sharded(e, false)) return 1;
         if (launch_day_sharded(e, true)) return 1;
         e->launches += (int64_t)n_days * SHARD_LAUNCHES_PER_DAY(G);
@@ -941,56 +891,28 @@ extern "C" int rb_step(rb_engine *e, int32_t n_days) {
         e->day += n_days;
         return 0;
     }
-    if (e->run_ctas) {      // few replicas: one persistent cooperative kernel for the whole step
-        CK(cudaEventRecord(e->ev0, e->stream));
-        cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof cfg);
-        cfg.gridDim = dim3(e->run_ctas, R); cfg.blockDim = dim3(RUN_THREADS); cfg.stream = e->stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeCooperative; at[0].val.cooperative = 1;      // the teams' barriers need every CTA resident
-        cfg.attrs = at; cfg.numAttrs = 1;
-        CK(cudaLaunchKernelEx(&cfg, k_run, G, (int)n_days, e->run_boundary_ctas));
-        e->launches++;
-        CK(cudaEventRecord(e->ev1, e->stream));
-        if (check_launches(e)) return 1;
-        e->day += n_days;
-        return 0;
-    }
-    if (e->n_groups > 1) {
-        CK(cudaEventRecord(e->ev0, e->stream));
-        launch_boundary(e, 0, R, e->stream, G); e->launches++;
-        CK(cudaEventRecord(e->ev_fork, e->stream));
-        for (int g = 0; g < e->n_groups; g++) {
-            ReplicaGroup &q = e->grp[g];
-            CK(cudaStreamWaitEvent(q.stream, e->ev_fork, 0));
-            int mid = n_days - 1;
-            if (g > 0 && mid > 0) CK(cudaStreamWaitEvent(q.stream, e->grp[g - 1].ev_stagger, 0));     // half a day behind the previous group
-            if (mid > 0) { launch_group_segment(e, q, g + 1 < e->n_groups); mid -= 1; e->launches += 4; }
-            while (mid >= GRAPH_DAYS) { CK(cudaGraphLaunch(q.graph[0], q.stream)); mid -= GRAPH_DAYS; e->launches += 4 * GRAPH_DAYS; }
-            while (mid > 0) { CK(cudaGraphLaunch(q.graph[1], q.stream)); mid -= 1; e->launches += 4; }
-            Eng Gq = G; Gq.r0 = q.r0;
-            launch_k(e, k_sweep, dim3(q.sweep_blocks, q.R), SW_THREADS, q.stream, Gq);
-            launch_k(e, k_expose, dim3(q.list_blocks, q.R), EX_THREADS, q.stream, Gq);
-            launch_k(e, k_resolve<false>, dim3(q.resolve_blocks, q.R), 256, q.stream, Gq, true);
-            launch_boundary(e, 1, q.R, q.stream, Gq);
-            e->launches += 4;
-            CK(cudaEventRecord(q.ev_join, q.stream));
-            CK(cudaStreamWaitEvent(e->stream, q.ev_join, 0));
-        }
-        CK(cudaEventRecord(e->ev1, e->stream));
-        if (check_launches(e)) return 1;
-        e->day += n_days;
-        return 0;
-    }
+    const int ng = e->n_groups;
     CK(cudaEventRecord(e->ev0, e->stream));
     launch_boundary(e, 0, R, e->stream, G); e->launches++;
-    int mid = n_days - 1;
-    while (mid >= GRAPH_DAYS) { CK(cudaGraphLaunch(e->graph[0], e->stream)); mid -= GRAPH_DAYS; e->launches += 4 * GRAPH_DAYS; }
-    while (mid > 0) { CK(cudaGraphLaunch(e->graph[1], e->stream)); mid -= 1; e->launches += 4; }
-    launch_k(e, k_sweep, dim3(e->sweep_blocks, R), SW_THREADS, e->stream, G);
-    launch_k(e, k_expose, dim3(e->list_blocks, R), EX_THREADS, e->stream, G);
-    launch_k(e, k_resolve<false>, dim3(e->resolve_blocks, R), 256, e->stream, G, true);
-    launch_boundary(e, 1, R, e->stream, G);
-    e->launches += 4;
+    if (ng > 1) CK(cudaEventRecord(e->ev_fork, e->stream));
+    for (int g = 0; g < ng; g++) {
+        ReplicaGroup &q = e->grp[g];
+        int mid = n_days - 1;
+        if (ng > 1) {
+            CK(cudaStreamWaitEvent(q.stream, e->ev_fork, 0));
+            if (g > 0 && mid > 0) CK(cudaStreamWaitEvent(q.stream, e->grp[g - 1].ev_stagger, 0));     // half a day behind the previous group
+            if (mid > 0) { launch_group_segment(e, q, g + 1 < ng); mid -= 1; e->launches += 4; }
+        }
+        while (mid >= GRAPH_DAYS) { CK(cudaGraphLaunch(q.graph[0], q.stream)); mid -= GRAPH_DAYS; e->launches += 4 * GRAPH_DAYS; }
+        while (mid > 0) { CK(cudaGraphLaunch(q.graph[1], q.stream)); mid -= 1; e->launches += 4; }
+        Eng Gq = G; Gq.r0 = q.r0;
+        launch_k(e, k_sweep, dim3(q.sweep_blocks, q.R), SW_THREADS, q.stream, Gq);
+        launch_k(e, k_expose, dim3(q.list_blocks, q.R), EX_THREADS, q.stream, Gq);
+        launch_k(e, k_resolve<false>, dim3(q.resolve_blocks, q.R), 256, q.stream, Gq, true);
+        launch_boundary(e, 1, q.R, q.stream, Gq);
+        e->launches += 4;
+        if (ng > 1) { CK(cudaEventRecord(q.ev_join, q.stream)); CK(cudaStreamWaitEvent(e->stream, q.ev_join, 0)); }
+    }
     CK(cudaEventRecord(e->ev1, e->stream));
     if (check_launches(e)) return 1;
     e->day += n_days;
@@ -1048,17 +970,14 @@ extern "C" int rb_step_timed(rb_engine *e, int32_t n_days, float *ms_per_kernel,
     struct Span { cudaEvent_t a, b; int k; };
     std::vector<Span> spans;
     auto mark = [&](cudaStream_t st) { cudaEvent_t x; cudaEventCreate(&x); cudaEventRecord(x, st); return x; };
-    // one group without streams of its own when the engine runs ungrouped
-    ReplicaGroup whole; whole.r0 = 0; whole.R = R; whole.sweep_blocks = e->sweep_blocks; whole.list_blocks = e->list_blocks;
-    whole.resolve_blocks = e->resolve_blocks; whole.stream = e->stream;
-    const int ng = e->n_groups > 1 ? e->n_groups : 1;
+    const int ng = e->n_groups;
     CK(cudaEventRecord(e->ev0, e->stream));
     { cudaEvent_t a = mark(e->stream); launch_boundary(e, 0, R, e->stream, G); spans.push_back({a, mark(e->stream), 0}); e->launches++; }
     if (ng > 1) CK(cudaEventRecord(e->ev_fork, e->stream));
     for (int d = 0; d < n_days; d++) {
         const bool last = d == n_days - 1;
         for (int g = 0; g < ng; g++) {
-            ReplicaGroup &q = ng > 1 ? e->grp[g] : whole;
+            ReplicaGroup &q = e->grp[g];
             if (ng > 1 && d == 0) {
                 CK(cudaStreamWaitEvent(q.stream, e->ev_fork, 0));
                 if (g > 0 && n_days > 1) CK(cudaStreamWaitEvent(q.stream, e->grp[g - 1].ev_stagger, 0));

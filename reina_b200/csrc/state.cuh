@@ -128,9 +128,10 @@ struct RepCtr {
     alignas(128) int32_t drain_det[RB_MAX_AGES];  // detections of an early queue drain, per age, booked at the next day boundary
     alignas(128) uint32_t n_l0;
     uint32_t n_l1, n_edges;
+    // an unused line that keeps RepCtr's layout: rb_save_state stores RepCtr raw (StateHeader::ctr_bytes checks its size),
+    // so blobs saved by earlier builds still load, and the kernels' field offsets stay as built
+    alignas(128) uint32_t reserved[2];
     // wide day boundary (boundary.cuh, Team): grid barrier word on its own line, today's verdict, per-CTA scan totals
-    alignas(128) unsigned int run_bar;            // k_run: barrier word of the replica's whole team
-    unsigned int run_exit;                        // k_run: CTAs that have left the final barrier
     alignas(128) unsigned int wide_bar;
     alignas(128) uint32_t wide_day;
     int32_t wide_mp[WIDE_MAX_CTAS][4];

@@ -226,34 +226,3 @@ def test_initial_population_condition(cuda_lib, oracle_lib):
     cpu = helpers.make_context(oracle_lib, seed=500, **kw)
     cpu.run(30)
     assert np.array_equal(gpu.series(0, 30)[0], cpu.series(0, 30)[0])
-
-
-@pytest.mark.parametrize('wide', [False, True])
-def test_persistent_run_kernel(cuda_lib, oracle_lib, monkeypatch, wide):
-    """RB_PERSISTENT=1: the whole run of a few replicas as ONE cooperative kernel (run.cuh, k_run) -- a team of co-resident
-    CTAs per replica walking through the phases of day after day behind its own barrier -- against the oracle: every
-    intervention type with a saturated tiny hospital, stepping in chunks, three replicas side by side; `wide` forces the
-    day boundary onto a sub-team of CTAs on every day."""
-    monkeypatch.setenv('RB_PERSISTENT', '1')
-    monkeypatch.setenv('RB_RUN_CTAS', '12')
-    if wide:
-        monkeypatch.setenv('RB_WIDE_MIN', '0')
-        monkeypatch.setenv('RB_WIDE_CTAS', '8')
-    counts = helpers.small_population(80000)
-    v = helpers.inputs.default_variables()
-    v['hospital_beds'], v['icu_units'] = 25, 3
-    kw = dict(variables=v, age_count_override=counts, interventions=helpers.stress_interventions())
-    gpu, cpu = _pair(cuda_lib, oracle_lib, seed=11, **kw)
-    launches0 = gpu._engine.launch_count()
-    _run_and_compare(gpu, cpu, 120, chunk=40)
-    # one k_run per chunk, plus a guide build per mobility epoch met while planning and the list flushes of read_agents;
-    # the per-phase kernels would have taken 1 + 4 x 120 launches
-    assert gpu._engine.launch_count() - launches0 <= 3 + 16
-    ens = helpers.make_context(cuda_lib, seed=40, n_replicas=3, **kw)
-    ens.run(100)
-    rows = ens.series(0, 100)
-    for r in range(3):
-        ref = helpers.make_context(oracle_lib, seed=40 + r, **kw)
-        ref.run(100)
-        assert np.array_equal(rows[r], ref.series(0, 100)[0]), 'replica %d differs' % r
-        assert np.array_equal(ens._engine.read_agents(r), ref._engine.read_agents(0))

@@ -21,20 +21,5 @@ rm -f $O/day92_k_resolve_R256.ncu-rep $O/day92_k_between_R256.ncu-rep
 for R in 256 32 1; do python tools/kern_times.py $R; done > $O/kernel_times_isolated.txt 2>&1
 python tools/group_exp.py --replicas 256 --configs 1:100,2:100,4:50,4:100,8:50 --steps 3 > $O/group_experiment.txt 2>&1
 python tools/group_exp.py --replicas 32 --configs 1:100,2:100,4:50,8:50 --steps 3 >> $O/group_experiment.txt 2>&1
-cat > /tmp/single.py <<'P'
-import os, sys, numpy as np
-sys.path.insert(0, '.')
-import bench
-R = int(sys.argv[1])
-ctx = bench.make_context(bench.workload_spec('hus'), R, 0, 180, seed=1)
-ms = []
-for s in range(5):
-    ctx.reset(60 + s); ctx.run(180)
-    if s >= 2: ms.append(ctx._engine.last_step_ms())
-print('R=%d RB_PERSISTENT=%s RB_RUN_CTAS=%s: %.3f ms per 180 days = %.1f us/day' % (R, os.environ.get('RB_PERSISTENT'), os.environ.get('RB_RUN_CTAS'), np.mean(ms), np.mean(ms) / 180 * 1e3), flush=True)
-P
-for cfg in "0 -" "1 16" "1 64" "1 148"; do set -- $cfg; RB_PERSISTENT=$1 RB_RUN_CTAS=$2 python /tmp/single.py 1; done > $O/persistent_kernel.txt 2>&1
-for cfg in "0 -" "1 9"; do set -- $cfg; RB_PERSISTENT=$1 RB_RUN_CTAS=$2 python /tmp/single.py 32; done >> $O/persistent_kernel.txt 2>&1
-RB_PERSISTENT=1 RB_RUN_CTAS=148 python tools/run_phases.py 1 >> $O/persistent_kernel.txt 2>&1
-cat $O/persistent_kernel.txt $O/group_experiment.txt
+cat $O/group_experiment.txt
 ls -la $O
