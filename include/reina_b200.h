@@ -312,6 +312,34 @@ int rb_branch(rb_engine *e, const int32_t *src, const uint32_t *seed);
  * reference counterpart. */
 int rb_read_seeds(rb_engine *e, uint32_t *out);
 
+/* ---- Moving replicas between engines and GPUs (no reference counterpart).
+ * A replica record is a header (magic, version, n_agents, Npad, n_ages, row_len, max_days, sus_words, cap_queue, the
+ * agent-record and counter sizes of this build, and the day) followed by one replica's slice of every part of the
+ * rb_save_state blob, in its order: packed words, agent records, both bitmaps, counters (with the sweep-order keys),
+ * both test queues, the stats rows [max_days + 1][row_len] and the replica's row of the seed history.  Written into a
+ * slot of an engine built from the same inputs and at the same day, a record continues exactly as the replica it came
+ * from would have, drawing with the seed the import gives it from today on (the record's own seed: the same future).
+ *   rb_replica_bytes       the size of one record, header included
+ *   rb_export_replicas     out[n][rb_replica_bytes] = records of replicas idx[0..n)
+ *   rb_import_replicas     writes n records (in, n * rb_replica_bytes bytes) into slots slot[0..n) with seeds seed[j]
+ *   rb_copy_replicas       replicas src_idx[j] of engine src into slots dst_slot[j] of engine dst (another engine of this
+ *                          process, on the same device or another one), device to device without staging
+ *   rb_comm_move_replicas  a collective over the engine's NCCL communicator (rb_comm_init): this rank sends replicas
+ *                          send_idx[i] to ranks send_peer[i] and receives into slots recv_slot[j] from ranks recv_peer[j],
+ *                          directly between the state arrays.  Every rank calls it with the same global plan; between two
+ *                          ranks the k-th replica sent is the k-th received.
+ * Refused (return 1, rb_last_error) with the engines left usable: a record or engine of another shape, build or day, an
+ * index, slot or peer out of range, a slot written twice, a slot that is also a source of the same call, the same
+ * engine as source and destination, and population-sharded engines.  Each waits for every stream of the engines
+ * involved first.  Contact tables and the schedule are inputs, not state: the caller keeps them equal.  CUDA library
+ * only. */
+int64_t rb_replica_bytes(rb_engine *e);
+int rb_export_replicas(rb_engine *e, int32_t n, const int32_t *idx, void *out, int64_t capacity);
+int rb_import_replicas(rb_engine *e, int32_t n, const int32_t *slot, const uint32_t *seed, const void *in, int64_t n_bytes);
+int rb_copy_replicas(rb_engine *dst, rb_engine *src, int32_t n, const int32_t *src_idx, const int32_t *dst_slot, const uint32_t *seed);
+int rb_comm_move_replicas(rb_engine *e, int32_t n_send, const int32_t *send_idx, const int32_t *send_peer,
+                          int32_t n_recv, const int32_t *recv_slot, const int32_t *recv_peer, const uint32_t *recv_seed);
+
 /* Measurement aids of the CUDA library (tools/phase_run.py): flag 9 makes the day-boundary kernels record the cycles
  * they spend per phase; rb_debug_phase_cycles reads the 16 accumulated counters of one replica.  No effect on results. */
 void rb_debug_flag(rb_engine *e, int32_t flag);

@@ -95,13 +95,16 @@ TX_SYMBOLS = ['transmission_len', 'transmission_stats', 'read_infection_days']
 SX_SYMBOLS = ['transmission_settings_len', 'transmission_settings', 'read_infection_places']
 # branching replicas from the current state; CPU reference: tests/oracle_branch.c (which includes the above)
 BRANCH_SYMBOLS = ['branch', 'read_seeds']
+# replica records moved between engines; CPU reference: tests/oracle_migrate.c (which includes the above).  The NCCL move
+# is CUDA only.
+MIGRATE_SYMBOLS = ['replica_bytes', 'export_replicas', 'import_replicas', 'copy_replicas']
 # exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes', 'comm_move_replicas'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS + MIGRATE_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -194,11 +197,14 @@ class Library:
             f['debug_phase_cycles'].argtypes = [vp, C.c_int32, C.c_void_p]
             f['copied_bytes'].argtypes = [vp, C.c_int32]
             f['copied_bytes'].restype = C.c_int64
+            i32p = C.POINTER(C.c_int32)
+            f['comm_move_replicas'].argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, i32p, i32p, C.POINTER(C.c_uint32)]
         self.f = f
         if prefix == 'rb_':
             self.bind_transmission()
             self.bind_settings()
             self.bind_branch()
+            self.bind_migrate()
 
     def bind_transmission(self):
         """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
@@ -228,6 +234,17 @@ class Library:
             f[name] = getattr(self.dll, self.prefix + name)
         f['branch'].argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_uint32)]
         f['read_seeds'].argtypes = [vp, C.POINTER(C.c_uint32)]
+
+    def bind_migrate(self):
+        """Bind the replica-record entry points (like bind_transmission)."""
+        f, vp, i32p = self.f, C.c_void_p, C.POINTER(C.c_int32)
+        for name in MIGRATE_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['replica_bytes'].argtypes = [vp]
+        f['replica_bytes'].restype = C.c_int64
+        f['export_replicas'].argtypes = [vp, C.c_int32, i32p, vp, C.c_int64]
+        f['import_replicas'].argtypes = [vp, C.c_int32, i32p, C.POINTER(C.c_uint32), vp, C.c_int64]
+        f['copy_replicas'].argtypes = [vp, vp, C.c_int32, i32p, i32p, C.POINTER(C.c_uint32)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -461,6 +478,43 @@ class Engine:
         out = np.empty((self.n_replicas, self.cfg.max_days + 1), dtype=np.uint32)
         self.lib.check(self.lib.f['read_seeds'](self.h, _ptr(out, C.c_uint32)), 'read_seeds')
         return out
+
+    # -- replica records (rb_replica_bytes / rb_export_replicas / rb_import_replicas / rb_copy_replicas) ----------
+    def replica_bytes(self):
+        return int(self.lib.f['replica_bytes'](self.h))
+
+    def export_replicas(self, idx):
+        """uint8 [n, replica_bytes]: the records of replicas idx."""
+        i = np.ascontiguousarray(idx, dtype=np.int32).ravel()
+        out = np.empty((i.size, self.replica_bytes()), dtype=np.uint8)
+        self.lib.check(self.lib.f['export_replicas'](self.h, i.size, _ptr(i, C.c_int32), out.ctypes.data, out.size), 'export_replicas')
+        return out
+
+    def import_replicas(self, slots, seeds, records):
+        s = np.ascontiguousarray(slots, dtype=np.int32).ravel()
+        k = np.ascontiguousarray(seeds, dtype=np.uint32).ravel()
+        b = np.ascontiguousarray(records, dtype=np.uint8)
+        assert s.shape == k.shape
+        self.lib.check(self.lib.f['import_replicas'](self.h, s.size, _ptr(s, C.c_int32), _ptr(k, C.c_uint32), b.ctypes.data, b.size),
+                       'import_replicas')
+
+    def copy_replicas_from(self, src, src_idx, slots, seeds):
+        """Replicas src_idx of Engine `src` into slots of this engine (rb_copy_replicas)."""
+        i = np.ascontiguousarray(src_idx, dtype=np.int32).ravel()
+        s = np.ascontiguousarray(slots, dtype=np.int32).ravel()
+        k = np.ascontiguousarray(seeds, dtype=np.uint32).ravel()
+        assert i.shape == s.shape == k.shape
+        self.lib.check(self.lib.f['copy_replicas'](self.h, src.h, i.size, _ptr(i, C.c_int32), _ptr(s, C.c_int32), _ptr(k, C.c_uint32)),
+                       'copy_replicas')
+
+    def comm_move_replicas(self, send_idx, send_peer, recv_slot, recv_peer, recv_seed):
+        """Collective replica moves over the engine's NCCL communicator (rb_comm_move_replicas)."""
+        a = [np.ascontiguousarray(x, dtype=np.int32).ravel() for x in (send_idx, send_peer, recv_slot, recv_peer)]
+        k = np.ascontiguousarray(recv_seed, dtype=np.uint32).ravel()
+        assert a[0].shape == a[1].shape and a[2].shape == a[3].shape == k.shape
+        self.lib.check(self.lib.f['comm_move_replicas'](self.h, a[0].size, _ptr(a[0], C.c_int32), _ptr(a[1], C.c_int32),
+                                                        a[2].size, _ptr(a[2], C.c_int32), _ptr(a[3], C.c_int32), _ptr(k, C.c_uint32)),
+                       'comm_move_replicas')
 
     def last_step_ms(self):
         return float(self.lib.f['last_step_ms'](self.h))

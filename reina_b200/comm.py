@@ -8,6 +8,10 @@ A communicator object has `rank`, `size`, `allreduce(x, op='sum'|'max')`, `allga
   * `EngineComm(engine)`     NCCL over NVLink through the engine handle (rb_comm_allreduce / rb_comm_allgather);
   * tests supply their own adapter over a CPU process group with the same five members (tests/helpers.py).
 
+A communicator may also have `sendrecv({peer: bytes}) -> {peer: bytes}`, a collective in which every rank sends its
+payloads and receives what the others sent it: ensemble.particle_filter moves replica records through it when the
+communicator is not the engine's own EngineComm (which moves them device to device, rb_comm_move_replicas).
+
 `connect(engine)` builds the right one from the launcher's environment (RANK / WORLD_SIZE, as torchrun sets them).
 """
 import os

@@ -1,5 +1,7 @@
 // reina_b200 / csrc / branch.cuh
 // Branching replicas (rb_branch): replica j continues from the current state of replica src[j] with a seed of its own.
+// Moving replicas (rb_import_replicas / rb_copy_replicas / rb_comm_move_replicas) writes the same state with plain copies
+// and finishes with k_import_fixup and k_branch_rebuild.
 // Two keys make this exact without touching any per-day kernel: RepCtr::seed keys every draw, RepCtr::fkey keys the
 // replica's fixed sweep-order permutation.  The copy takes the source's fkey along with its state, so every sweep position
 // already stored (test queue, capacity events, perm) stays valid, and the new seed changes only the draws of the days to
@@ -75,6 +77,18 @@ __global__ void k_branch_rebuild(Eng G, const int32_t *src) {
         if (h & H_QUEUED) h |= H_DET;
         list_add(G, r, c, cur, (uint32_t)a, h);
     }
+}
+
+// After replica records were written into slots slot[0..n) (rb_import_replicas, rb_copy_replicas,
+// rb_comm_move_replicas): one CTA per slot gives it its seed -- in the counters and in the seed history from `today` on
+// (the days before came with the record) -- and zeroes its list counters for k_branch_rebuild.
+__global__ void k_import_fixup(Eng G, uint32_t *seed_of_day, const int32_t *slot, const uint32_t *seed, int today) {
+    const int j = slot[blockIdx.x];
+    const uint32_t s = seed[blockIdx.x];
+    const size_t M = (size_t)G.max_days + 1;
+    if (threadIdx.x == 0) G.ctr[j].seed = s;
+    for (size_t d = (size_t)today + threadIdx.x; d < M; d += blockDim.x) seed_of_day[(size_t)j * M + d] = s;
+    for (size_t i = threadIdx.x; i < 2 * (size_t)G.n_seg; i += blockDim.x) G.seg_n[2 * (size_t)G.n_seg * j + i] = make_uint2(0u, 0u);
 }
 
 // Seed history of a fresh population (rb_create, rb_reset: seed + r on every day) or of a version-2 checkpoint (the

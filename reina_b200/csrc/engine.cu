@@ -17,7 +17,8 @@
 //   setup.cuh     set_initial_state, initialisation, contact-row guide, snapshot, ensemble moments, samplers
 //   transmission.cuh  k_transmission: cohort / offspring / generation-interval tables from the infection tree (not per day);
 //                 k_transmission_settings: the same tree by place of infection and age group
-//   branch.cuh    k_branch_copy / k_branch_rebuild: replicas continue from another replica's current state (rb_branch)
+//   branch.cuh    k_branch_copy / k_branch_rebuild: replicas continue from another replica's current state (rb_branch);
+//                 k_import_fixup: replica records written into slots (rb_import_replicas, rb_copy_replicas, rb_comm_move_replicas)
 //   this file     host side: engine handle, launch geometry, replica groups, CUDA graphs, NCCL binding (ensemble reduce,
 //                 sharded mode), the extern "C" entry points
 //
@@ -89,6 +90,7 @@ struct rb_engine {
     int32_t *d_tx;                      // [R][rb_transmission_len] tables of rb_transmission_stats, allocated by its first call
     int32_t *d_sx, *d_sx_epoch;         // [R][rb_transmission_settings_len] tables, [max_days + 1] epoch of each day: allocated by the first settings call
     int32_t *d_branch;                  // [R] sources then [R] seeds of rb_branch, allocated by its first call
+    int32_t *d_move;                    // [3R] slots, seeds and rebuild markers of a replica import, allocated by the first one
     uint32_t *seed_of_day;              // [R][max_days + 1] seed history (branch.cuh)
 };
 
@@ -101,6 +103,10 @@ struct NcclApi {
     ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t);
     ncclResult_t (*CommDestroy)(ncclComm_t);
     const char *(*GetErrorString)(ncclResult_t);
+    ncclResult_t (*Send)(const void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t);
+    ncclResult_t (*Recv)(void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t);
+    ncclResult_t (*GroupStart)(void);
+    ncclResult_t (*GroupEnd)(void);
 };
 static NcclApi g_nccl;
 static int load_nccl() {
@@ -116,7 +122,12 @@ static int load_nccl() {
     g_nccl.AllReduce = (ncclResult_t(*)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t))dlsym(h, "ncclAllReduce");
     g_nccl.CommDestroy = (ncclResult_t(*)(ncclComm_t))dlsym(h, "ncclCommDestroy");
     g_nccl.GetErrorString = (const char *(*)(ncclResult_t))dlsym(h, "ncclGetErrorString");
-    if (!g_nccl.GetUniqueId || !g_nccl.CommInitRank || !g_nccl.AllGather || !g_nccl.AllReduce || !g_nccl.CommDestroy || !g_nccl.GetErrorString) {
+    g_nccl.Send = (ncclResult_t(*)(const void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t))dlsym(h, "ncclSend");
+    g_nccl.Recv = (ncclResult_t(*)(void *, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t))dlsym(h, "ncclRecv");
+    g_nccl.GroupStart = (ncclResult_t(*)(void))dlsym(h, "ncclGroupStart");
+    g_nccl.GroupEnd = (ncclResult_t(*)(void))dlsym(h, "ncclGroupEnd");
+    if (!g_nccl.GetUniqueId || !g_nccl.CommInitRank || !g_nccl.AllGather || !g_nccl.AllReduce || !g_nccl.CommDestroy || !g_nccl.GetErrorString ||
+        !g_nccl.Send || !g_nccl.Recv || !g_nccl.GroupStart || !g_nccl.GroupEnd) {
         snprintf(g_err, sizeof g_err, "libnccl.so.2 lacks a required symbol"); return 1;
     }
     g_nccl.dl = h;
@@ -201,7 +212,7 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     rb_engine *e = new rb_engine();
     e->cfg = *cfg; e->day = 0; e->last_ms = 0; e->launches = 0; e->h2d_bytes = 0; e->d2h_bytes = 0; e->have_graphs = false; e->comm = nullptr; e->comm_rank = 0; e->comm_size = 1; e->sharded = false; e->merge_blocks = 1;
     e->has_ipc = false; e->h_stage = nullptr; e->n_stage = 0; e->n_groups = 1; e->wide_ctas = 1; e->n_peer_open = 0; e->launch_err = cudaSuccess; e->shard_timing = getenv("RB_SHARD_TIMING") != nullptr;
-    e->xepoch = 0; e->d_xepoch = nullptr; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr; e->d_branch = nullptr;
+    e->xepoch = 0; e->d_xepoch = nullptr; e->d_tx = nullptr; e->d_sx = nullptr; e->d_sx_epoch = nullptr; e->d_branch = nullptr; e->d_move = nullptr;
     { int lo = 0, hi = 0; CK(cudaDeviceGetStreamPriorityRange(&lo, &hi)); e->prio_high = hi; e->prio = (cfg->n_replicas >= 32 && cfg->n_replicas < 128) ? 1 : 0; if (const char *s = getenv("RB_PRIO")) e->prio = atoi(s); }
     CK(cudaStreamCreateWithFlags(&e->stream, cudaStreamNonBlocking));
     CK(cudaEventCreate(&e->ev0)); CK(cudaEventCreate(&e->ev1));
@@ -1411,4 +1422,197 @@ extern "C" int rb_read_seeds(rb_engine *e, uint32_t *out) {
     CK(cudaMemcpy(out, e->seed_of_day, bytes, cudaMemcpyDeviceToHost));
     e->d2h_bytes += (int64_t)bytes;
     return 0;
+}
+
+// ---------------------------------------------------------------- moving replicas between engines and GPUs (branch.cuh)
+// A replica record: this header, then the replica's slice of every state part, in the order of state_parts.  Every part
+// is [R][per-replica bytes], so a record is read and written with one plain copy per part, straight from and into the
+// state arrays.  The header holds what must match for the bytes to mean the same thing in another engine; the replica
+// count and the launch geometry need not (the active lists are rebuilt in the destination's own segments).
+struct ReplicaHeader {
+    uint64_t magic; int32_t version, n_agents, npad, n_ages, row_len, max_days, sus_words;
+    uint32_t cap_queue; int32_t rec_bytes, ctr_bytes, day, reserved[3];
+};
+static_assert(sizeof(ReplicaHeader) == 64, "ReplicaHeader is 64 bytes");
+#define REPLICA_MAGIC 0x3150455252414e49ull    // "INARREP1"
+
+static ReplicaHeader replica_header(rb_engine *e) {
+    const Eng &G = e->G;
+    ReplicaHeader h; memset(&h, 0, sizeof h);
+    h.magic = REPLICA_MAGIC; h.version = 1; h.n_agents = G.N; h.npad = G.Npad; h.n_ages = G.n_ages; h.row_len = G.row_len;
+    h.max_days = G.max_days; h.sus_words = G.sus_words; h.cap_queue = G.cap_queue;
+    h.rec_bytes = (int32_t)sizeof(AgentRec); h.ctr_bytes = (int32_t)sizeof(RepCtr); h.day = e->day;
+    return h;
+}
+
+// replica r's slice of every part of state_parts
+static std::vector<StatePart> replica_parts(rb_engine *e, int r) {
+    std::vector<StatePart> v = state_parts(e);
+    for (StatePart &p : v) { p.bytes /= (size_t)e->G.R; p.dev = (uint8_t *)p.dev + (size_t)r * p.bytes; }
+    return v;
+}
+
+extern "C" int64_t rb_replica_bytes(rb_engine *e) {
+    size_t n = sizeof(ReplicaHeader);
+    for (const StatePart &p : replica_parts(e, 0)) n += p.bytes;
+    return (int64_t)n;
+}
+
+// The checks every move makes of the engine that is written.  Returns 1 with g_err set.
+static int check_slots(rb_engine *e, const char *fn, int32_t n, const int32_t *slot) {
+    const int R = e->G.R;
+    if (e->sharded) { snprintf(g_err, sizeof g_err, "%s: not available in population-sharded mode", fn); return 1; }
+    if (n < 0 || n > R) { snprintf(g_err, sizeof g_err, "%s: %d slots for %d replicas", fn, n, R); return 1; }
+    std::vector<char> seen(R, 0);
+    for (int j = 0; j < n; j++) {
+        if (slot[j] < 0 || slot[j] >= R) { snprintf(g_err, sizeof g_err, "%s: slot[%d] = %d is not a replica (0 .. %d)", fn, j, slot[j], R - 1); return 1; }
+        if (seen[slot[j]]) { snprintf(g_err, sizeof g_err, "%s: slot %d is written twice", fn, slot[j]); return 1; }
+        seen[slot[j]] = 1;
+    }
+    return 0;
+}
+static int check_sources(rb_engine *e, const char *fn, int32_t n, const int32_t *idx) {
+    if (e->sharded) { snprintf(g_err, sizeof g_err, "%s: not available in population-sharded mode", fn); return 1; }
+    if (n < 0) { snprintf(g_err, sizeof g_err, "%s: negative count", fn); return 1; }
+    for (int j = 0; j < n; j++)
+        if (idx[j] < 0 || idx[j] >= e->G.R) { snprintf(g_err, sizeof g_err, "%s: index[%d] = %d is not a replica (0 .. %d)", fn, j, idx[j], e->G.R - 1); return 1; }
+    return 0;
+}
+// Records of another shape, build or day than engine e's (h.day against e's day first: the more useful message).
+static int check_header(rb_engine *e, const char *fn, const ReplicaHeader &h, int j) {
+    ReplicaHeader w = replica_header(e);
+    if (h.magic == w.magic && h.day != w.day) { snprintf(g_err, sizeof g_err, "%s: record %d is of day %d, the engine is at day %d", fn, j, h.day, w.day); return 1; }
+    if (memcmp(&h, &w, sizeof h) != 0) { snprintf(g_err, sizeof g_err, "%s: record %d was made by an engine of another shape (agents / ages / max_days / build)", fn, j); return 1; }
+    return 0;
+}
+
+// After the bytes of n records were queued on e->stream into slots slot[0..n): the seeds, the seed history from today
+// on, then the active lists and perm of the written slots (k_branch_rebuild with -1 marking them).  Waits for the end.
+static int finish_import(rb_engine *e, int32_t n, const int32_t *slot, const uint32_t *seed) {
+    const Eng &G = e->G;
+    const int R = G.R;
+    if (n > 0) {
+        if (!e->d_move && dalloc(e, &e->d_move, 3 * (size_t)R)) return 1;
+        std::vector<int32_t> h(2 * (size_t)n + R);
+        for (int j = 0; j < n; j++) { h[j] = slot[j]; h[n + j] = (int32_t)seed[j]; }
+        for (int r = 0; r < R; r++) h[2 * n + r] = r;
+        for (int j = 0; j < n; j++) h[2 * n + slot[j]] = -1;
+        CK(cudaMemcpyAsync(e->d_move, h.data(), sizeof(int32_t) * h.size(), cudaMemcpyHostToDevice, e->stream));
+        e->h2d_bytes += (int64_t)sizeof(int32_t) * h.size();
+        k_import_fixup<<<n, 256, 0, e->stream>>>(G, e->seed_of_day, e->d_move, (const uint32_t *)(e->d_move + n), e->day);
+        k_branch_rebuild<<<dim3(e->sweep_blocks, R), 256, 0, e->stream>>>(G, e->d_move + 2 * n);
+        e->launches += 2;
+        CK(cudaGetLastError());
+    }
+    CK(cudaStreamSynchronize(e->stream));
+    return 0;
+}
+
+// the day counters live in the active lists: into the packed words first, so that a record carries them (as rb_save_state)
+static int flush_for_export(rb_engine *e) {
+    if (sync_all_streams(e)) return 1;
+    k_flush_lists<<<dim3(e->sweep_blocks, e->G.R), 256, 0, e->stream>>>(e->G); e->launches++;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int rb_export_replicas(rb_engine *e, int32_t n, const int32_t *idx, void *out, int64_t capacity) {
+    CK(cudaSetDevice(e->cfg.device));
+    if (check_sources(e, "rb_export_replicas", n, idx)) return 1;
+    const int64_t rb = rb_replica_bytes(e);
+    if (capacity < rb * n) { snprintf(g_err, sizeof g_err, "rb_export_replicas: buffer of %lld bytes, need %lld", (long long)capacity, (long long)(rb * n)); return 1; }
+    if (flush_for_export(e)) return 1;
+    const ReplicaHeader h = replica_header(e);
+    uint8_t *o = (uint8_t *)out;
+    for (int j = 0; j < n; j++) {
+        memcpy(o, &h, sizeof h); o += sizeof h;
+        for (const StatePart &p : replica_parts(e, idx[j])) { CK(cudaMemcpyAsync(o, p.dev, p.bytes, cudaMemcpyDeviceToHost, e->stream)); o += p.bytes; }
+    }
+    CK(cudaStreamSynchronize(e->stream));
+    e->d2h_bytes += (rb - (int64_t)sizeof h) * n;
+    return 0;
+}
+
+extern "C" int rb_import_replicas(rb_engine *e, int32_t n, const int32_t *slot, const uint32_t *seed, const void *in, int64_t n_bytes) {
+    CK(cudaSetDevice(e->cfg.device));
+    if (check_slots(e, "rb_import_replicas", n, slot)) return 1;
+    const int64_t rb = rb_replica_bytes(e);
+    if (n_bytes != rb * n) { snprintf(g_err, sizeof g_err, "rb_import_replicas: %lld bytes for %d records of %lld", (long long)n_bytes, n, (long long)rb); return 1; }
+    const uint8_t *o = (const uint8_t *)in;
+    for (int j = 0; j < n; j++) {
+        ReplicaHeader h; memcpy(&h, o + rb * j, sizeof h);
+        if (check_header(e, "rb_import_replicas", h, j)) return 1;
+    }
+    if (sync_all_streams(e)) return 1;
+    for (int j = 0; j < n; j++) {
+        o += sizeof(ReplicaHeader);
+        for (const StatePart &p : replica_parts(e, slot[j])) { CK(cudaMemcpyAsync(p.dev, o, p.bytes, cudaMemcpyHostToDevice, e->stream)); o += p.bytes; }
+    }
+    e->h2d_bytes += (rb - (int64_t)sizeof(ReplicaHeader)) * n;
+    return finish_import(e, n, slot, seed);
+}
+
+extern "C" int rb_copy_replicas(rb_engine *dst, rb_engine *src, int32_t n, const int32_t *src_idx, const int32_t *dst_slot, const uint32_t *seed) {
+    if (dst == src) { snprintf(g_err, sizeof g_err, "rb_copy_replicas: source and destination are the same engine (rb_branch copies within one)"); return 1; }
+    if (check_sources(src, "rb_copy_replicas", n, src_idx) || check_slots(dst, "rb_copy_replicas", n, dst_slot)) return 1;
+    if (check_header(dst, "rb_copy_replicas", replica_header(src), 0)) return 1;
+    CK(cudaSetDevice(src->cfg.device));
+    if (flush_for_export(src)) return 1;
+    CK(cudaStreamSynchronize(src->stream));
+    CK(cudaSetDevice(dst->cfg.device));
+    if (sync_all_streams(dst)) return 1;
+    const int ds = src->cfg.device, dd = dst->cfg.device;
+    for (int j = 0; j < n; j++) {
+        const std::vector<StatePart> s = replica_parts(src, src_idx[j]), d = replica_parts(dst, dst_slot[j]);
+        for (size_t k = 0; k < s.size(); k++) {
+            if (ds == dd) CK(cudaMemcpyAsync(d[k].dev, s[k].dev, s[k].bytes, cudaMemcpyDeviceToDevice, dst->stream));
+            else CK(cudaMemcpyPeerAsync(d[k].dev, dd, s[k].dev, ds, s[k].bytes, dst->stream));
+        }
+    }
+    return finish_import(dst, n, dst_slot, seed);
+}
+
+// Collective over the engine's communicator.  Every rank first checks its own arguments, then the ranks exchange their
+// headers and verdicts (one small all-gather), so that a plan or shape one rank refuses is refused by all of them and
+// nobody is left waiting in a send.  Sends and receives of every part then go in one NCCL group.
+extern "C" int rb_comm_move_replicas(rb_engine *e, int32_t n_send, const int32_t *send_idx, const int32_t *send_peer,
+                                     int32_t n_recv, const int32_t *recv_slot, const int32_t *recv_peer, const uint32_t *recv_seed) {
+    const char *fn = "rb_comm_move_replicas";
+    CK(cudaSetDevice(e->cfg.device));
+    if (!e->comm || e->sharded) { snprintf(g_err, sizeof g_err, "%s: needs the ensemble communicator of rb_comm_init (and no population-sharded mode)", fn); return 1; }
+    const int K = e->comm_size, me = e->comm_rank;
+    int bad = check_sources(e, fn, n_send, send_idx) || check_slots(e, fn, n_recv, recv_slot);
+    for (int i = 0; i < n_send && !bad; i++)
+        if (send_peer[i] < 0 || send_peer[i] >= K || send_peer[i] == me) { snprintf(g_err, sizeof g_err, "%s: send_peer[%d] = %d is not another rank", fn, i, send_peer[i]); bad = 1; }
+    for (int j = 0; j < n_recv && !bad; j++) {
+        if (recv_peer[j] < 0 || recv_peer[j] >= K || recv_peer[j] == me) { snprintf(g_err, sizeof g_err, "%s: recv_peer[%d] = %d is not another rank", fn, j, recv_peer[j]); bad = 1; }
+        for (int i = 0; i < n_send && !bad; i++)
+            if (send_idx[i] == recv_slot[j]) { snprintf(g_err, sizeof g_err, "%s: replica %d is both sent and written", fn, recv_slot[j]); bad = 1; }
+    }
+    struct Hello { ReplicaHeader h; int32_t bad, pad[15]; };
+    static_assert(sizeof(Hello) == 128, "Hello is one 128-byte record");
+    Hello mine; memset(&mine, 0, sizeof mine);
+    mine.h = replica_header(e); mine.bad = bad;
+    if (sync_all_streams(e)) return 1;
+    void *d; bool temp;
+    if (comm_scratch(e, sizeof(Hello) * K, &d, &temp)) return 1;
+    std::vector<Hello> all(K);
+    CK(cudaMemcpyAsync((Hello *)d + me, &mine, sizeof mine, cudaMemcpyHostToDevice, e->stream));
+    NK(g_nccl.AllGather((Hello *)d + me, d, sizeof(Hello), ncclChar, e->comm, e->stream));
+    CK(cudaMemcpyAsync(all.data(), d, sizeof(Hello) * K, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    if (temp) cudaFree(d);
+    if (bad) return 1;
+    for (int k = 0; k < K; k++) {
+        if (all[k].bad) { snprintf(g_err, sizeof g_err, "%s: rank %d refused the plan", fn, k); return 1; }
+        if (memcmp(&all[k].h, &mine.h, sizeof mine.h) != 0) { snprintf(g_err, sizeof g_err, "%s: rank %d holds an engine of another shape, build or day", fn, k); return 1; }
+    }
+    if (n_send > 0 && flush_for_export(e)) return 1;
+    NK(g_nccl.GroupStart());
+    for (int i = 0; i < n_send; i++)
+        for (const StatePart &p : replica_parts(e, send_idx[i])) NK(g_nccl.Send(p.dev, p.bytes, ncclChar, send_peer[i], e->comm, e->stream));
+    for (int j = 0; j < n_recv; j++)
+        for (const StatePart &p : replica_parts(e, recv_slot[j])) NK(g_nccl.Recv(p.dev, p.bytes, ncclChar, recv_peer[j], e->comm, e->stream));
+    NK(g_nccl.GroupEnd());
+    return finish_import(e, n_recv, recv_slot, recv_seed);
 }

@@ -12,6 +12,7 @@ import math
 
 import numpy as np
 
+from . import model as _model
 from .comm import LocalComm
 
 
@@ -223,6 +224,32 @@ def assign_slots(counts):
     return src.astype(np.int32)
 
 
+def migration_plan(counts, n_ranks):
+    """The global `source` for resampling counts over n_ranks x R replicas (rank k holds global indices k R .. k R + R - 1)
+    that moves the fewest replicas between ranks: a replica with counts >= 1 keeps its slot, a rank's extra copies fill
+    that rank's own dropped slots first (in increasing order), and only the remaining dropped slots are filled across
+    ranks, with the remaining extra copies, both in increasing global order.  That is sum_k max(0, dropped_k - extras_k)
+    moves, the least any plan needs.  source[source[j]] == source[j]; with n_ranks = 1 it is assign_slots(counts)."""
+    c = np.asarray(counts, dtype=np.int64)
+    if c.ndim != 1 or (c < 0).any() or c.sum() != c.size:
+        raise ValueError('counts must be >= 0 and sum to their number')
+    if n_ranks < 1 or c.size % n_ranks:
+        raise ValueError('%d counts do not split over %d ranks' % (c.size, n_ranks))
+    R = c.size // n_ranks
+    src = np.arange(c.size)
+    holes, extras = [], []
+    for k in range(n_ranks):
+        ck = c[k * R:(k + 1) * R]
+        extra = np.repeat(np.arange(R), np.maximum(ck - 1, 0)) + k * R
+        dropped = np.flatnonzero(ck == 0) + k * R
+        m = min(extra.size, dropped.size)
+        src[dropped[:m]] = extra[:m]
+        holes.append(dropped[m:])
+        extras.append(extra[m:])
+    src[np.concatenate(holes)] = np.concatenate(extras)
+    return src.astype(np.int32)
+
+
 def _lgamma(x):
     return np.vectorize(math.lgamma, otypes=[np.float64])(x)
 
@@ -266,47 +293,126 @@ def _logsumexp(x):
     return m + math.log(np.exp(x - m).sum()) if np.isfinite(m) else m
 
 
-def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0):
-    """Sequential importance resampling of the replicas of ONE Context against observed counts.
+def _gather(comm, x):
+    """[ranks * len(x), ...] of every rank's x (uint32 travels as int32: not every collective backend has uint32)."""
+    x = np.ascontiguousarray(x)
+    if comm.size == 1:
+        return x
+    if x.dtype == np.uint32:
+        return np.asarray(comm.allgather(x.view(np.int32))).view(np.uint32).reshape((-1,) + x.shape[1:])
+    return np.asarray(comm.allgather(x)).reshape((-1,) + x.shape[1:])
+
+
+def _move_replicas(ctxs, comm, rank, src, seeds, R):
+    """Apply the global plan `src` with the global `seeds` to this process's Contexts (ctxs[i] holds global replicas
+    (rank + i) R ..): Context.branch for sources on the same Context, copy_replicas_from between the Contexts of this
+    process, rb_comm_move_replicas over the engine's own communicator, else host records through comm.sendrecv."""
+    from .comm import EngineComm
+    N = src.size
+    for i, c in enumerate(ctxs):                      # sources on the same Context
+        g0 = (rank + i) * R
+        loc = np.arange(R, dtype=np.int32)
+        same = (src[g0:g0 + R] // R) == (g0 // R)
+        loc[same] = src[g0:g0 + R][same] - g0
+        if (loc != np.arange(R)).any():
+            c.branch(loc, seeds[g0:g0 + R])
+    cross = [j for j in range(N) if src[j] // R != j // R]            # increasing global destination order
+    if not cross:
+        return
+    if comm.size == 1:                                # the Contexts of this process
+        pairs = {}
+        for j in cross:
+            pairs.setdefault((j // R, src[j] // R), []).append(j)
+        for (kd, ks), js in pairs.items():
+            js = np.array(js)
+            ctxs[kd].copy_replicas_from(ctxs[ks], src[js] % R, js % R, seeds[js])
+        return
+    ctx = ctxs[0]
+    send = [j for j in cross if src[j] // R == rank]
+    recv = [j for j in cross if j // R == rank]
+    if isinstance(comm, EngineComm) and comm.engine is ctx._engine:
+        ctx._engine.comm_move_replicas([src[j] % R for j in send], [j // R for j in send], [j % R for j in recv],
+                                       [src[j] // R for j in recv], seeds[recv])
+        ctx._state_day = -1
+        return
+    if not hasattr(comm, 'sendrecv'):
+        raise TypeError('particle_filter: moving replicas between ranks needs the engine\'s own EngineComm or a '
+                        'communicator with sendrecv({peer: bytes}) -> {peer: bytes}')
+    out = {}
+    for j in send:
+        out.setdefault(j // R, []).append(src[j] % R)
+    payload = {p: ctx.export_replicas(idx).tobytes() for p, idx in out.items()}
+    got = comm.sendrecv(payload)
+    by_peer = {}
+    for j in recv:
+        by_peer.setdefault(src[j] // R, []).append(j)
+    for p, js in sorted(by_peer.items()):
+        js = np.array(js)
+        ctx.import_replicas(js % R, np.frombuffer(got[p], dtype=np.uint8).reshape(len(js), -1), seeds[js])
+
+
+def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0, comm=None):
+    """Sequential importance resampling of an ensemble against observed counts: the replicas of ONE Context, of a list
+    of Contexts of this process, or of every rank's Context (`comm`, one Context per rank), filtered as ONE set of
+    particles.  Global replica g = k R + r is replica r of Context / rank k; every Context holds R replicas.
 
     observations = {day: {name: count}}: `name` is an ATTRS name summed over the age groups ('in_ward', 'in_icu',
     'dead', 'all_detected', ...) or a row_layout() column.  The observation of day d is compared with stats row d, the
     state before the d-th iterate() (what generate_state() returns at ctx.day == d); the days must not lie before
     ctx.day.  The likelihood of a replica is a negative binomial with mean equal to its count and dispersion k
     (`dispersion`), or Poisson (model='poisson'); several names on one day are independent.  After each observation
-    day the weights are updated, and when the effective sample size falls below ess_threshold * R -- and always at the
-    last observation -- the replicas are resampled systematically (systematic_resample with a Generator seeded by
-    `seed`) and copied on the device with Context.branch (assign_slots): every copy continues with a fresh seed.
+    day the log-likelihoods of all replicas are gathered (comm.allgather, or over the list), the weights are updated, and
+    when the effective sample size falls below ess_threshold * K R -- and always at the last observation -- the replicas
+    are resampled systematically (systematic_resample with a Generator seeded by `seed`, the same on every rank) and
+    copied with the plan of migration_plan, which moves the fewest replicas between Contexts.  Every copy continues with
+    a fresh seed: Context.branch's rule over the union of every Context's seed history, in global order.  Copies on one
+    Context use Context.branch; between Contexts of this process copy_replicas_from; between ranks
+    rb_comm_move_replicas when `comm` is the engine's own EngineComm, else host records through comm.sendrecv.  A list
+    of Contexts together with a communicator of several ranks is refused.
 
-    The Context is left at the last observation day, equally weighted, so run(), series(), moments() and
+    The Contexts are left at the last observation day, equally weighted, so run(), series(), moments() and
     percentile_bands() give the forecast from there.  The rows of days before it are the paths of the surviving
     replicas' ancestors: for early days few distinct paths remain (they degenerate), so read the past from the filter's
-    weights at each day, not from the returned ensemble.  Resampling across GPUs (moving replica state between ranks) is
-    not provided: every rank filters its own replicas.
+    weights at each day, not from the returned ensemble.
 
-    Returns a dict: log_evidence (the sum over the observation days of the log mean incremental weight), days[k],
-    ess[k] (before resampling), resampled[k], ancestors[k, R] (the branch source of step k, the identity where nothing
-    was resampled) and loglik[k, R].  Raises ValueError naming the day if no replica can explain an observation (every
-    weight zero)."""
-    R = ctx.n_replicas
+    Returns a dict, the same on every rank: log_evidence (the sum over the observation days of the log mean incremental
+    weight), days[k], ess[k] (before resampling), resampled[k], ancestors[k, K R] (the global source of step k, the
+    identity where nothing was resampled), loglik[k, K R] and seeds[k, K R] (every replica's seed from that day on).
+    Raises ValueError naming the day if no replica can explain an observation (every weight zero)."""
+    ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
+    comm = comm or LocalComm()
+    if not ctxs or (len(ctxs) > 1 and comm.size > 1):
+        raise ValueError('particle_filter: one Context per rank, or a list of Contexts without a communicator of several ranks')
+    R, c0 = ctxs[0].n_replicas, ctxs[0]
+    if any(c.n_replicas != R or c.day != c0.day for c in ctxs):
+        raise ValueError('particle_filter: the Contexts must hold as many replicas each and be at the same day')
+    rank = comm.rank if comm.size > 1 else 0
+    N = R * len(ctxs) * comm.size
     days = sorted(int(d) for d in observations)
-    if days and (days[0] < ctx.day or days[-1] > ctx.max_days):
-        raise ValueError('observation days must lie in [ctx.day, max_days] = [%d, %d]' % (ctx.day, ctx.max_days))
+    if days and (days[0] < c0.day or days[-1] > c0.max_days):
+        raise ValueError('observation days must lie in [ctx.day, max_days] = [%d, %d]' % (c0.day, c0.max_days))
     rng = np.random.default_rng(seed)
-    logw = np.full(R, -math.log(R))
+    logw = np.full(N, -math.log(N))
     out = dict(log_evidence=0.0, days=np.array(days, dtype=np.int64), ess=np.zeros(len(days)),
-               resampled=np.zeros(len(days), dtype=bool), ancestors=np.zeros((len(days), R), dtype=np.int32),
-               loglik=np.zeros((len(days), R)))
+               resampled=np.zeros(len(days), dtype=bool), ancestors=np.zeros((len(days), N), dtype=np.int32),
+               loglik=np.zeros((len(days), N)), seeds=np.zeros((len(days), N), dtype=np.uint32))
+    hist = None
     for k, d in enumerate(days):
-        if d > ctx.day:
-            ctx.run(d - ctx.day)
-        ctx._engine.snapshot()
-        ctx._engine.sync()
-        ctx._state_day = ctx.day
-        rows = ctx._engine.read_stats(d, 1)[:, 0].astype(np.float64)
-        ll = np.zeros(R)
-        for name, y in observations[d].items():
-            ll += log_likelihood(_model_counts(ctx, rows, name), y, model, dispersion)
+        parts = []
+        for c in ctxs:
+            if d > c.day:
+                c.run(d - c.day)
+            c._engine.snapshot()
+            c._engine.sync()
+            c._state_day = c.day
+            rows = c._engine.read_stats(d, 1)[:, 0].astype(np.float64)
+            ll = np.zeros(R)
+            for name, y in observations[d].items():
+                ll += log_likelihood(_model_counts(c, rows, name), y, model, dispersion)
+            parts.append(ll)
+        ll = _gather(comm, np.concatenate(parts))
+        if hist is None:                              # the seed history of every replica, in global order
+            hist = _gather(comm, np.concatenate([c._engine.read_seeds() for c in ctxs]))
         post = logw + ll
         total = _logsumexp(post)
         if not np.isfinite(total):
@@ -315,12 +421,18 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
         logw = post - total
         w = np.exp(logw)
         ess = 1.0 / (w * w).sum()
-        src = np.arange(R, dtype=np.int32)
-        if ess < ess_threshold * R or k == len(days) - 1:
-            src = assign_slots(systematic_resample(w, rng))
-            if (src != np.arange(R)).any():
-                ctx.branch(src)
-            logw = np.full(R, -math.log(R))
+        src = np.arange(N, dtype=np.int32)
+        if ess < ess_threshold * N or k == len(days) - 1:
+            src = migration_plan(systematic_resample(w, rng), N // R)
+            changed = np.flatnonzero(src != np.arange(N))
+            seeds = hist[:, d].astype(np.int64)
+            seeds[changed] = _model.fresh_seeds(hist, changed.size)
+            if changed.size:
+                _move_replicas(ctxs, comm, rank, src, seeds.astype(np.uint32), R)
+                hist[:, :d] = hist[src, :d]
+                hist[:, d:] = seeds.astype(np.uint32)[:, None]
+            logw = np.full(N, -math.log(N))
             out['resampled'][k] = True
         out['ess'][k], out['ancestors'][k], out['loglik'][k] = ess, src, ll
+        out['seeds'][k] = hist[:, d]
     return out

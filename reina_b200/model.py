@@ -239,6 +239,21 @@ def ncontact_cdf(nr_contacts_by_age):
 # ---------------------------------------------------------------------------------------------------
 # Context
 # ---------------------------------------------------------------------------------------------------
+def fresh_seeds(hist, n):
+    """n seeds none of which occurs in the seed history `hist` (any shape): counting up from its largest seed, skipping
+    used ones (modulo 2^32).  Context.branch gives these to the replicas whose state it changes."""
+    h = np.asarray(hist, dtype=np.uint32)
+    used = set(h.ravel().tolist())
+    nxt = int(h.max()) + 1 if h.size else 0
+    out = np.zeros(n, dtype=np.int64)
+    for j in range(n):
+        while (nxt & 0xFFFFFFFF) in used:
+            nxt += 1
+        out[j] = nxt & 0xFFFFFFFF
+        used.add(int(out[j]))
+    return out
+
+
 class Context:
     """model.Context (main.pyx:1746-2101) over the CUDA engine."""
 
@@ -575,22 +590,77 @@ class Context:
         src = np.full(R, int(source), dtype=np.int64) if np.ndim(source) == 0 else np.asarray(source, dtype=np.int64)
         if src.shape != (R,):
             raise ValueError('source must be one int or %d ints' % R)
-        hist = self._engine.read_seeds()
         if seeds is None:
+            hist = self._engine.read_seeds()
             seeds = hist[:, self.day].copy()
-            used = set(hist.ravel().tolist())
-            nxt = int(hist.max()) + 1
-            for j in np.flatnonzero(src != np.arange(R)):
-                while (nxt & 0xFFFFFFFF) in used:
-                    nxt += 1
-                seeds[j] = nxt & 0xFFFFFFFF
-                used.add(int(seeds[j]))
+            changed = np.flatnonzero(src != np.arange(R))
+            seeds[changed] = fresh_seeds(hist, changed.size)
         seeds = np.asarray(seeds, dtype=np.int64)
         if seeds.shape != (R,) or (seeds < 0).any() or (seeds > 0xFFFFFFFF).any():
             raise ValueError('seeds must be %d unsigned 32-bit ints' % R)
         self._engine.branch(src, seeds.astype(np.uint32))
         self._state_day = -1
         return seeds.astype(np.uint32)
+
+    # -- moving replicas between Contexts, engines and GPUs --------------------------------------------------------
+    def _check_movable(self, other):
+        """Refuses two Contexts the engines cannot tell apart but a moved replica would notice: a different schedule of
+        the days run so far, or different contact tables of those days' epochs (inputs, not state)."""
+        if other.day != self.day:
+            raise ValueError('the Contexts are at days %d and %d' % (self.day, other.day))
+        if len(self._plan) < self.day or len(other._plan) < other.day or \
+                any(bytes(a) != bytes(b) for a, b in zip(self._plan[:self.day], other._plan[:other.day])):
+            raise ValueError('the Contexts ran different schedules (interventions) so far')
+        for ep in sorted({0} | {dp.table_epoch for dp in self._plan[:self.day]}):
+            a, b = self._tables.get(ep), other._tables.get(ep)
+            if a is None or b is None or a.keys() != b.keys() or any(not np.array_equal(a[k], b[k]) for k in a):
+                raise ValueError('the Contexts use different contact tables (epoch %d)' % ep)
+
+    def _import_seeds(self, slots, seeds, foreign_hist):
+        """The seeds of written slots: as given, or (None) seeds neither this engine nor the incoming replicas' seed
+        histories ever used -- Context.branch's rule over both."""
+        if seeds is None:
+            hist = self._engine.read_seeds()
+            seeds = fresh_seeds(np.concatenate([hist, foreign_hist.reshape(-1, hist.shape[1])]), len(slots))
+        seeds = np.asarray(seeds, dtype=np.int64)
+        if seeds.shape != (len(slots),) or (seeds < 0).any() or (seeds > 0xFFFFFFFF).any():
+            raise ValueError('seeds must be %d unsigned 32-bit ints' % len(slots))
+        return seeds.astype(np.uint32)
+
+    def export_replicas(self, idx):
+        """Replica records (rb_export_replicas) of replicas `idx`: uint8 [len(idx), record bytes].  Everything a replica
+        needs to continue -- agents, infection tree, test queue, counters, sweep-order keys, stats rows so far and its
+        seed history, which ends every record -- for import_replicas() into a Context built the same way, at the same day,
+        in this process or another one."""
+        return self._engine.export_replicas(np.atleast_1d(np.asarray(idx, dtype=np.int64)))
+
+    def import_replicas(self, slots, records, seeds=None):
+        """Write export_replicas() records into `slots` (rb_import_replicas): each slot continues from its record with
+        seed seeds[j] from today on (the record's own seed: exactly as the replica it came from).  seeds None: seeds
+        that neither this engine nor the records' seed histories have used.  Returns the seeds given."""
+        slots = np.atleast_1d(np.asarray(slots, dtype=np.int64))
+        rec = np.ascontiguousarray(records, dtype=np.uint8).reshape(len(slots), -1) if len(slots) else np.zeros((0, 0), np.uint8)
+        foreign = rec[:, rec.shape[1] - 4 * (self.max_days + 1):].copy().view(np.uint32) if len(slots) else np.zeros((0, self.max_days + 1), np.uint32)
+        seeds = self._import_seeds(slots, seeds, foreign)
+        self._engine.import_replicas(slots, seeds, rec)
+        self._state_day = -1
+        return seeds
+
+    def copy_replicas_from(self, other, src_idx, slots, seeds=None):
+        """Replicas src_idx of Context `other` (another Context of this process, on this GPU or another one) into
+        `slots` of this one, device to device (rb_copy_replicas); seeds as in import_replicas().  Returns the seeds
+        given."""
+        if other is self:
+            raise ValueError('copy_replicas_from: the same Context (Context.branch copies within one)')
+        self._check_movable(other)
+        src_idx = np.atleast_1d(np.asarray(src_idx, dtype=np.int64))
+        slots = np.atleast_1d(np.asarray(slots, dtype=np.int64))
+        if src_idx.shape != slots.shape:
+            raise ValueError('src_idx and slots differ in length')
+        seeds = self._import_seeds(slots, seeds, other._engine.read_seeds() if seeds is None else np.zeros((0, self.max_days + 1), np.uint32))
+        self._engine.copy_replicas_from(other._engine, src_idx, slots, seeds)
+        self._state_day = -1
+        return seeds
 
     def replica_seeds(self):
         """The seed every replica draws with from today on (random_seed + r until a branch changes it)."""
