@@ -82,7 +82,8 @@ typedef struct rb_config {
     int32_t max_days;      /* capacity of the per-day stats buffer */
     int32_t n_import_classes;           /* imported_infection_ages, main.pyx:1376-1384 */
     int32_t device;        /* CUDA device ordinal (ignored by the oracle) */
-    float contact_capacity;  /* capacity of the per-day contact work list, in units of n_agents (0 = default) */
+    float contact_capacity;  /* capacity of the per-day contact work list, in units of n_agents (0 = default); the list of
+                                the day's transmissions (n_agents / 8) takes the same factor */
     int32_t reserved[4];
 } rb_config;
 
@@ -311,6 +312,20 @@ int rb_branch(rb_engine *e, const int32_t *src, const uint32_t *seed);
 /* out[R][max_days + 1]: the draw seed of every replica on every day (days after today: the seed in force now).  No
  * reference counterpart. */
 int rb_read_seeds(rb_engine *e, uint32_t *out);
+
+/* ---- Per-replica transmission scale (no reference counterpart).
+ * Replica r's scale f_r multiplies the transmission probability of every contact its infectors make, every variant and
+ * every place: min(1, f_r p) with p = did_infect's (source infectiousness * susceptibility) * infectiousness multiplier;
+ * masks act afterwards as before.  It takes effect from the next rb_step and is part of the replica's state: rb_branch,
+ * replica records, rb_copy_replicas, rb_comm_move_replicas and rb_save_state / rb_load_state carry it; rb_create and
+ * rb_reset give 1, and blobs and records of earlier builds load with 1.  The engine stores f - 1 in float and multiplies by
+ * 1 + (f - 1), so every f = 1 computes exactly what an engine without scales does.
+ *   rb_set_transmission_scale   scale[R]: every value finite and in (0, 16], else refused (return 1, rb_last_error) with
+ *                               nothing changed.  Waits for every stream of the engine first.  Allowed in
+ *                               population-sharded mode, where every rank makes the same call.
+ *   rb_read_transmission_scale  out[R] = 1 + (f - 1) as stored: f itself for 0.5 <= f <= 2. */
+int rb_set_transmission_scale(rb_engine *e, const float *scale);
+int rb_read_transmission_scale(rb_engine *e, float *out);
 
 /* ---- Moving replicas between engines and GPUs (no reference counterpart).
  * A replica record is a header (magic, version, n_agents, Npad, n_ages, row_len, max_days, sus_words, cap_queue, the

@@ -98,13 +98,15 @@ BRANCH_SYMBOLS = ['branch', 'read_seeds']
 # replica records moved between engines; CPU reference: tests/oracle_migrate.c (which includes the above).  The NCCL move
 # is CUDA only.
 MIGRATE_SYMBOLS = ['replica_bytes', 'export_replicas', 'import_replicas', 'copy_replicas']
+# the per-replica transmission scale; CPU reference: tests/oracle_tscale.c (which includes the above)
+TSCALE_SYMBOLS = ['set_transmission_scale', 'read_transmission_scale']
 # exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes', 'comm_move_replicas'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS + MIGRATE_SYMBOLS
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes', 'comm_move_replicas'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS + MIGRATE_SYMBOLS + TSCALE_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -205,6 +207,7 @@ class Library:
             self.bind_settings()
             self.bind_branch()
             self.bind_migrate()
+            self.bind_tscale()
 
     def bind_transmission(self):
         """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
@@ -245,6 +248,14 @@ class Library:
         f['export_replicas'].argtypes = [vp, C.c_int32, i32p, vp, C.c_int64]
         f['import_replicas'].argtypes = [vp, C.c_int32, i32p, C.POINTER(C.c_uint32), vp, C.c_int64]
         f['copy_replicas'].argtypes = [vp, vp, C.c_int32, i32p, i32p, C.POINTER(C.c_uint32)]
+
+    def bind_tscale(self):
+        """Bind rb_set_transmission_scale / rb_read_transmission_scale (like bind_transmission)."""
+        f, vp = self.f, C.c_void_p
+        for name in TSCALE_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['set_transmission_scale'].argtypes = [vp, C.POINTER(C.c_float)]
+        f['read_transmission_scale'].argtypes = [vp, C.POINTER(C.c_float)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -515,6 +526,17 @@ class Engine:
         self.lib.check(self.lib.f['comm_move_replicas'](self.h, a[0].size, _ptr(a[0], C.c_int32), _ptr(a[1], C.c_int32),
                                                         a[2].size, _ptr(a[2], C.c_int32), _ptr(a[3], C.c_int32), _ptr(k, C.c_uint32)),
                        'comm_move_replicas')
+
+    def set_transmission_scale(self, scale):
+        """float32 [n_replicas]: every replica's transmission scale, in force from the next step."""
+        s = np.ascontiguousarray(scale, dtype=np.float32)
+        assert s.shape == (self.n_replicas,)
+        self.lib.check(self.lib.f['set_transmission_scale'](self.h, _ptr(s, C.c_float)), 'set_transmission_scale')
+
+    def read_transmission_scale(self):
+        out = np.empty(self.n_replicas, dtype=np.float32)
+        self.lib.check(self.lib.f['read_transmission_scale'](self.h, _ptr(out, C.c_float)), 'read_transmission_scale')
+        return out
 
     def last_step_ms(self):
         return float(self.lib.f['last_step_ms'](self.h))

@@ -44,7 +44,7 @@ __device__ __forceinline__ void expose_survivors(const Eng &G, int r, RepCtr *c,
         if ((__ldg(&sus[t >> 5]) >> (t & 31)) & 1u) {
             const int tage = tb->susc_uniform[age][row] ? (int)tb->lo_age[age][row]
                                                         : age_in_band(G, (int32_t)t, tb->lo_age[age][row], tb->hi_age[age][row]);
-            const float pr = (si * v->tab[RB_T_SUSCEPTIBILITY][tage]) * v->infectiousness_multiplier;
+            const float pr = ((si * v->tab[RB_T_SUSCEPTIBILITY][tage]) * v->infectiousness_multiplier) * (1.0f + c->tscale_m1);
             if (((double)y.y * (1.0 / 4294967296.0)) * (double)kq < (double)pr * 256.0) {
                 ok = true;
                 const float mp = tb->mask_p[age][row];
@@ -105,7 +105,9 @@ __device__ __forceinline__ void expose_cta(const Eng &G, const int r, const uint
             const rb_variant *v = &G.variants[(it.y >> 20) & 3u];
             float si = v->iot[(it.y >> 14) & 31u];
             if ((it.y >> 19) & 1u) si = si * v->p_asymptomatic_infection;
-            const float p_upper = (si * v->reserved[0]) * v->infectiousness_multiplier;
+            // the replica's transmission scale f (RepCtr::tscale_m1) multiplies p and p_upper alike: float products are
+            // monotone, so pr <= p_upper still holds, and with kq = 256 a pr >= 1 always passes, which is min(1, f p)
+            const float p_upper = ((si * v->reserved[0]) * v->infectiousness_multiplier) * (1.0f + c->tscale_m1);
             kq = (int)(p_upper * 256.0f) + 1;
             if (kq > 256) kq = 256;
             const u32x4 x = philox(c->seed, it.x, day, PU_CONTACT | (grp << 8), 0);

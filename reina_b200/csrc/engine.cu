@@ -240,7 +240,8 @@ extern "C" int rb_create(const rb_config *cfg, const int32_t *age_counts, const 
     }
     float cc = cfg->contact_capacity > 0 ? cfg->contact_capacity : 1.0f;
     G.cap_items = pow2_at_least((uint64_t)((double)N * cc) + 4096);
-    G.cap_succ = pow2_at_least((uint64_t)N / 8 + 4096);
+    // the day's transmissions grow with its contacts (a transmission scale above 1 grows both), so they take the same factor
+    G.cap_succ = pow2_at_least((uint64_t)((double)((uint64_t)N / 8) * cc) + 4096);
     G.cap_events = pow2_at_least((uint64_t)N / 16 + 2048);
     G.cap_queue = pow2_at_least((uint64_t)N / 8 + 2048);
     const size_t RN = (size_t)R * G.Npad;
@@ -1421,6 +1422,32 @@ extern "C" int rb_read_seeds(rb_engine *e, uint32_t *out) {
     const size_t bytes = sizeof(uint32_t) * (size_t)e->G.R * (e->G.max_days + 1);
     CK(cudaMemcpy(out, e->seed_of_day, bytes, cudaMemcpyDeviceToHost));
     e->d2h_bytes += (int64_t)bytes;
+    return 0;
+}
+
+// ---------------------------------------------------------------- per-replica transmission scale (RepCtr::tscale_m1)
+// One strided copy into (or out of) the tscale_m1 word of every replica's counter block, as rb_problem reads `problem`.
+extern "C" int rb_set_transmission_scale(rb_engine *e, const float *scale) {
+    CK(cudaSetDevice(e->cfg.device));
+    const int R = e->G.R;
+    std::vector<float> m1(R);
+    for (int r = 0; r < R; r++) {
+        if (!(scale[r] > 0.0f && scale[r] <= 16.0f)) { snprintf(g_err, sizeof g_err, "rb_set_transmission_scale: scale[%d] = %g is not in (0, 16]", r, (double)scale[r]); return 1; }
+        m1[r] = scale[r] - 1.0f;
+    }
+    if (sync_all_streams(e)) return 1;
+    CK(cudaMemcpy2DAsync(&e->G.ctr[0].tscale_m1, sizeof(RepCtr), m1.data(), sizeof(float), sizeof(float), (size_t)R, cudaMemcpyHostToDevice, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    e->h2d_bytes += (int64_t)sizeof(float) * R;
+    return 0;
+}
+
+extern "C" int rb_read_transmission_scale(rb_engine *e, float *out) {
+    CK(cudaSetDevice(e->cfg.device));
+    if (sync_all_streams(e)) return 1;
+    CK(cudaMemcpy2D(out, sizeof(float), &e->G.ctr[0].tscale_m1, sizeof(RepCtr), sizeof(float), (size_t)e->G.R, cudaMemcpyDeviceToHost));
+    for (int r = 0; r < e->G.R; r++) out[r] = 1.0f + out[r];
+    e->d2h_bytes += (int64_t)sizeof(float) * e->G.R;
     return 0;
 }
 

@@ -128,9 +128,12 @@ struct RepCtr {
     alignas(128) int32_t drain_det[RB_MAX_AGES];  // detections of an early queue drain, per age, booked at the next day boundary
     alignas(128) uint32_t n_l0;
     uint32_t n_l1, n_edges;
-    // an unused line that keeps RepCtr's layout: rb_save_state stores RepCtr raw (StateHeader::ctr_bytes checks its size),
-    // so blobs saved by earlier builds still load, and the kernels' field offsets stay as built
-    alignas(128) uint32_t reserved[2];
+    // the replica's transmission scale f minus 1 (rb_set_transmission_scale; k_expose multiplies every transmission
+    // probability by 1 + tscale_m1), so that a zeroed RepCtr means f = 1 exactly.  It sits on the line that was unused
+    // until then: rb_save_state and replica records store RepCtr raw (their headers check its size), so the layout stays,
+    // blobs and records of earlier builds load with f = 1, and every copy of a replica's counters carries f along.
+    alignas(128) float tscale_m1;
+    uint32_t reserved;
     // wide day boundary (boundary.cuh, Team): grid barrier word on its own line, today's verdict, per-CTA scan totals
     alignas(128) unsigned int wide_bar;
     alignas(128) uint32_t wide_day;

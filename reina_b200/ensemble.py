@@ -351,7 +351,19 @@ def _move_replicas(ctxs, comm, rank, src, seeds, R):
         ctx.import_replicas(js % R, np.frombuffer(got[p], dtype=np.uint8).reshape(len(js), -1), seeds[js])
 
 
-def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0, comm=None):
+def _set_scales(ctxs, rank, R, scale):
+    """Each of this process's Contexts sets its slice of the global scales (ctxs[i] holds global replicas (rank + i) R ..)."""
+    for i, c in enumerate(ctxs):
+        g0 = (rank + i) * R
+        c.set_transmission_scale(scale[g0:g0 + R])
+
+
+# the range a filtered transmission scale is kept in: the engine accepts (0, 16]
+_LOG_SCALE_MIN, _LOG_SCALE_MAX = math.log(1.0 / 16.0), math.log(16.0)
+
+
+def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0, comm=None,
+                    transmission_prior=None, transmission_volatility=0.0):
     """Sequential importance resampling of an ensemble against observed counts: the replicas of ONE Context, of a list
     of Contexts of this process, or of every rank's Context (`comm`, one Context per rank), filtered as ONE set of
     particles.  Global replica g = k R + r is replica r of Context / rank k; every Context holds R replicas.
@@ -377,8 +389,19 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
 
     Returns a dict, the same on every rank: log_evidence (the sum over the observation days of the log mean incremental
     weight), days[k], ess[k] (before resampling), resampled[k], ancestors[k, K R] (the global source of step k, the
-    identity where nothing was resampled), loglik[k, K R] and seeds[k, K R] (every replica's seed from that day on).
-    Raises ValueError naming the day if no replica can explain an observation (every weight zero)."""
+    identity where nothing was resampled), loglik[k, K R] and seeds[k, K R] (every replica's seed from that day on), and
+    weights[k, K R] (normalised, before resampling).  Raises ValueError naming the day if no replica can explain an
+    observation (every weight zero).
+
+    transmission_prior = (median, log_sd) filters every replica's transmission scale f (Context.set_transmission_scale)
+    together with its state.  Before the first observation every global replica draws log f ~ N(log median, log_sd^2)
+    from the filter's Generator, in global order, the same on every rank.  At each observation day but the last, after
+    the weight update and any resampling (a copy arrives with its source's f), every replica takes a random-walk step
+    log f += transmission_volatility * sqrt(d_next - d) * eps, eps ~ N(0, 1), when the volatility is > 0.  log f is kept
+    in [log 1/16, log 16].  After the last observation there is no step: the forecast runs with the scales in force.  The
+    output then also holds transmission_scale[k, K R], the scales (float32, as set) the weights of day k judged:
+    weighted_quantiles(out['transmission_scale'][k], out['weights'][k], q) is the scale's posterior band at that day.
+    With transmission_prior None, transmission_scale is None and the Contexts' scales are never touched."""
     ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
     comm = comm or LocalComm()
     if not ctxs or (len(ctxs) > 1 and comm.size > 1):
@@ -395,7 +418,17 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
     logw = np.full(N, -math.log(N))
     out = dict(log_evidence=0.0, days=np.array(days, dtype=np.int64), ess=np.zeros(len(days)),
                resampled=np.zeros(len(days), dtype=bool), ancestors=np.zeros((len(days), N), dtype=np.int32),
-               loglik=np.zeros((len(days), N)), seeds=np.zeros((len(days), N), dtype=np.uint32))
+               loglik=np.zeros((len(days), N)), seeds=np.zeros((len(days), N), dtype=np.uint32),
+               weights=np.zeros((len(days), N)), transmission_scale=None)
+    logf = None
+    if transmission_prior is not None:
+        median, log_sd = (float(x) for x in transmission_prior)
+        if not (median > 0 and log_sd >= 0 and transmission_volatility >= 0):
+            raise ValueError('transmission_prior needs median > 0 and log_sd >= 0, and the volatility must be >= 0')
+        logf = np.clip(rng.normal(math.log(median), log_sd, N), _LOG_SCALE_MIN, _LOG_SCALE_MAX)
+        scale = np.exp(logf).astype(np.float32)
+        _set_scales(ctxs, rank, R, scale)
+        out['transmission_scale'] = np.zeros((len(days), N), dtype=np.float32)
     hist = None
     for k, d in enumerate(days):
         parts = []
@@ -421,6 +454,9 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
         logw = post - total
         w = np.exp(logw)
         ess = 1.0 / (w * w).sum()
+        out['weights'][k] = w
+        if logf is not None:
+            out['transmission_scale'][k] = scale
         src = np.arange(N, dtype=np.int32)
         if ess < ess_threshold * N or k == len(days) - 1:
             src = migration_plan(systematic_resample(w, rng), N // R)
@@ -435,4 +471,35 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
             out['resampled'][k] = True
         out['ess'][k], out['ancestors'][k], out['loglik'][k] = ess, src, ll
         out['seeds'][k] = hist[:, d]
+        if logf is not None:
+            logf, scale = logf[src], scale[src]           # the copies already carry their source's scale on the device
+            if k < len(days) - 1 and transmission_volatility > 0:
+                step = transmission_volatility * math.sqrt(days[k + 1] - d)
+                logf = np.clip(logf + step * rng.standard_normal(N), _LOG_SCALE_MIN, _LOG_SCALE_MAX)
+                scale = np.exp(logf).astype(np.float32)
+                _set_scales(ctxs, rank, R, scale)
     return out
+
+
+def weighted_quantiles(values, weights, q):
+    """Quantiles of weighted samples along the last axis: for each q, the smallest value whose share of the total weight
+    at or below it is >= q (the inverse of the weighted empirical distribution function; with equal weights
+    np.quantile(..., method='inverted_cdf')).  values and weights [..., N], weights >= 0 with a positive sum along the last
+    axis; q a number or a sequence in [0, 1].  Returns [...] for a number, [len(q), ...] for a sequence: e.g. the 5 / 50 /
+    95 % band of a particle filter's transmission scale at every observation day from out['transmission_scale'] and
+    out['weights']."""
+    x = np.asarray(values, dtype=np.float64)
+    if x.ndim == 0 or x.shape[-1] == 0:
+        raise ValueError('values need a last axis of at least one sample')
+    w = np.broadcast_to(np.asarray(weights, dtype=np.float64), x.shape)
+    if not np.isfinite(w).all() or (w < 0).any() or not (w.sum(-1) > 0).all():
+        raise ValueError('weights must be finite, >= 0 and not all 0 along the last axis')
+    qs = np.asarray(q, dtype=np.float64)
+    if ((qs < 0) | (qs > 1)).any():
+        raise ValueError('quantiles must lie in [0, 1]')
+    order = np.argsort(x, axis=-1, kind='stable')
+    xs, cw = np.take_along_axis(x, order, -1), np.cumsum(np.take_along_axis(w, order, -1), axis=-1)
+    cw = cw / cw[..., -1:]
+    idx = np.stack([np.minimum((cw < qi).sum(-1), x.shape[-1] - 1) for qi in np.atleast_1d(qs)])
+    res = np.take_along_axis(np.broadcast_to(xs, idx.shape[:1] + xs.shape), idx[..., None], -1)[..., 0]
+    return res[0] if qs.ndim == 0 else res

@@ -666,6 +666,24 @@ class Context:
         """The seed every replica draws with from today on (random_seed + r until a branch changes it)."""
         return self._engine.read_seeds()[:, self.day].copy()
 
+    def set_transmission_scale(self, values):
+        """Every replica's transmission scale f (rb_set_transmission_scale): one value for all replicas or n_replicas
+        values, each finite and in (0, 16].  Replica r's infectors then transmit with probability min(1, f_r p) where
+        they would with p, at every place and for every variant, from the next iterate() on.  The scale is part of the
+        replica's state: branch(), export / import, copy_replicas_from() and save_state() / load_state() carry it, and
+        reset() and a fresh Context give 1.  Refused values raise EngineError and change nothing."""
+        R = self.n_replicas
+        v = np.full(R, values, dtype=np.float64) if np.ndim(values) == 0 else np.asarray(values, dtype=np.float64)
+        if v.shape != (R,):
+            raise ValueError('transmission scale: one value or %d values' % R)
+        with np.errstate(over='ignore'):                  # a value beyond float32 becomes inf, which the engine refuses
+            self._engine.set_transmission_scale(v.astype(np.float32))
+
+    def transmission_scale(self):
+        """float32 [n_replicas]: the scales in force, as the engine applies them (1 + (f - 1) in float: f itself for
+        0.5 <= f <= 2)."""
+        return self._engine.read_transmission_scale()
+
     def row_layout(self):
         G = len(self.age_group_labels)
         names = ['%s[%s]' % (a, g) for a in ATTRS for g in self.age_group_labels]
