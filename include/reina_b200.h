@@ -327,6 +327,25 @@ int rb_read_seeds(rb_engine *e, uint32_t *out);
 int rb_set_transmission_scale(rb_engine *e, const float *scale);
 int rb_read_transmission_scale(rb_engine *e, float *out);
 
+/* ---- Per-replica severity scales (no reference counterpart).
+ * Replica r has three scales: severe s_r, critical c_r and fatal q_r.  Where an infection's severity is drawn
+ * (Disease.get_symptom_severity: transmissions, imports and rb_set_initial_state), the wild-type variant's conditional
+ * probabilities of the infected age become
+ *     sc' = min(sc s, max(sc, 1))   cc' = min(cc c, max(cc, 1))   fc' = min(fc q, max(fc, 1))   dohc' = min(dohc q, max(dohc, 1))
+ * and are used in place of the tables' in the same expressions.  A scaled probability passes 1 only where the table
+ * already does.  The fatal scale acts on both fatal paths; since FATAL is nested inside CRITICAL and every FATAL case dies
+ * outside hospital, raising it turns critical cases into deaths and in_icu falls.  dohc' = 1 divides by zero in
+ * (val - dohc) / (1 - dohc) exactly as the reference's expression would: -inf, a FATAL case.  rb_sample stays unscaled.
+ * Like the transmission scale, the scales are part of the replica's state, are stored as f - 1 (every f = 1 computes
+ * exactly what an engine without scales does), take effect from the next rb_step (rb_set_initial_state reads them when
+ * it runs), and rb_create / rb_reset give 1.
+ *   rb_set_severity_scale   scale[R][3] = (severe, critical, fatal): every value finite and in (0, 16], else refused
+ *                           (return 1, rb_last_error) with nothing changed.  Waits for every stream of the engine first.
+ *                           Allowed in population-sharded mode, where every rank makes the same call.
+ *   rb_read_severity_scale  out[R][3] = 1 + (f - 1) as stored. */
+int rb_set_severity_scale(rb_engine *e, const float *scale);
+int rb_read_severity_scale(rb_engine *e, float *out);
+
 /* ---- Moving replicas between engines and GPUs (no reference counterpart).
  * A replica record is a header (magic, version, n_agents, Npad, n_ages, row_len, max_days, sus_words, cap_queue, the
  * agent-record and counter sizes of this build, and the day) followed by one replica's slice of every part of the

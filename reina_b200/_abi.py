@@ -100,13 +100,15 @@ BRANCH_SYMBOLS = ['branch', 'read_seeds']
 MIGRATE_SYMBOLS = ['replica_bytes', 'export_replicas', 'import_replicas', 'copy_replicas']
 # the per-replica transmission scale; CPU reference: tests/oracle_tscale.c (which includes the above)
 TSCALE_SYMBOLS = ['set_transmission_scale', 'read_transmission_scale']
+# the per-replica severity scales; CPU reference: tests/oracle_sscale.c (which includes the above)
+SSCALE_SYMBOLS = ['set_severity_scale', 'read_severity_scale']
 # exported by the CUDA library only: population-sharded mode (the sequential CPU oracle has no ranks) and the rest below
 SHARD_SYMBOLS = ['shard_unique_id', 'shard_init', 'shard_init_local', 'shard_rank', 'shard_nranks', 'shard_message_bytes', 'shard_exchange',
                  # checkpoint / resume of the device-resident state
                  'state_bytes', 'save_state', 'load_state',
                  # ensemble communicator (NCCL), production-geometry timing, measurement aids
                  'comm_init', 'comm_rank', 'comm_size', 'comm_allreduce', 'comm_allgather', 'reduce_moments',
-                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes', 'comm_move_replicas'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS + MIGRATE_SYMBOLS + TSCALE_SYMBOLS
+                 'step_timed', 'debug_flag', 'debug_phase_cycles', 'copied_bytes', 'comm_move_replicas'] + TX_SYMBOLS + SX_SYMBOLS + BRANCH_SYMBOLS + MIGRATE_SYMBOLS + TSCALE_SYMBOLS + SSCALE_SYMBOLS
 SH_SHIFT = 12      # ownership stripes of 4096 agents, dealt round-robin over the ranks (engine.cu owns())
 
 
@@ -208,6 +210,7 @@ class Library:
             self.bind_branch()
             self.bind_migrate()
             self.bind_tscale()
+            self.bind_sscale()
 
     def bind_transmission(self):
         """Bind the transmission-statistics entry points (the CUDA library exports them; a test library that adds them
@@ -256,6 +259,14 @@ class Library:
             f[name] = getattr(self.dll, self.prefix + name)
         f['set_transmission_scale'].argtypes = [vp, C.POINTER(C.c_float)]
         f['read_transmission_scale'].argtypes = [vp, C.POINTER(C.c_float)]
+
+    def bind_sscale(self):
+        """Bind rb_set_severity_scale / rb_read_severity_scale (like bind_transmission)."""
+        f, vp = self.f, C.c_void_p
+        for name in SSCALE_SYMBOLS:
+            f[name] = getattr(self.dll, self.prefix + name)
+        f['set_severity_scale'].argtypes = [vp, C.POINTER(C.c_float)]
+        f['read_severity_scale'].argtypes = [vp, C.POINTER(C.c_float)]
 
     def check(self, rc, what):
         if rc != 0:
@@ -536,6 +547,17 @@ class Engine:
     def read_transmission_scale(self):
         out = np.empty(self.n_replicas, dtype=np.float32)
         self.lib.check(self.lib.f['read_transmission_scale'](self.h, _ptr(out, C.c_float)), 'read_transmission_scale')
+        return out
+
+    def set_severity_scale(self, scale):
+        """float32 [n_replicas, 3]: every replica's severe, critical and fatal scales, in force from the next step."""
+        s = np.ascontiguousarray(scale, dtype=np.float32)
+        assert s.shape == (self.n_replicas, 3)
+        self.lib.check(self.lib.f['set_severity_scale'](self.h, _ptr(s, C.c_float)), 'set_severity_scale')
+
+    def read_severity_scale(self):
+        out = np.empty((self.n_replicas, 3), dtype=np.float32)
+        self.lib.check(self.lib.f['read_severity_scale'](self.h, _ptr(out, C.c_float)), 'read_severity_scale')
         return out
 
     def last_step_ms(self):

@@ -1425,30 +1425,52 @@ extern "C" int rb_read_seeds(rb_engine *e, uint32_t *out) {
     return 0;
 }
 
-// ---------------------------------------------------------------- per-replica transmission scale (RepCtr::tscale_m1)
-// One strided copy into (or out of) the tscale_m1 word of every replica's counter block, as rb_problem reads `problem`.
-extern "C" int rb_set_transmission_scale(rb_engine *e, const float *scale) {
+// ---------------------------------------------------------------- per-replica scales (RepCtr::tscale_m1, sscale_m1)
+// `k` scales per replica, stored as f - 1 in `k` consecutive floats of every replica's counter block starting at `field`
+// (a member of G.ctr[0]).  One strided copy into (or out of) them, as rb_problem reads `problem`; every value is checked
+// before anything is written, so a refused call changes nothing.
+static int set_replica_scales(rb_engine *e, const char *fn, float *field, int k, const float *scale) {
     CK(cudaSetDevice(e->cfg.device));
     const int R = e->G.R;
-    std::vector<float> m1(R);
-    for (int r = 0; r < R; r++) {
-        if (!(scale[r] > 0.0f && scale[r] <= 16.0f)) { snprintf(g_err, sizeof g_err, "rb_set_transmission_scale: scale[%d] = %g is not in (0, 16]", r, (double)scale[r]); return 1; }
-        m1[r] = scale[r] - 1.0f;
+    std::vector<float> m1((size_t)R * k);
+    for (int i = 0; i < R * k; i++) {
+        if (!(scale[i] > 0.0f && scale[i] <= 16.0f)) {
+            if (k == 1) snprintf(g_err, sizeof g_err, "%s: scale[%d] = %g is not in (0, 16]", fn, i, (double)scale[i]);
+            else snprintf(g_err, sizeof g_err, "%s: scale[%d][%d] = %g is not in (0, 16]", fn, i / k, i % k, (double)scale[i]);
+            return 1;
+        }
+        m1[i] = scale[i] - 1.0f;
     }
     if (sync_all_streams(e)) return 1;
-    CK(cudaMemcpy2DAsync(&e->G.ctr[0].tscale_m1, sizeof(RepCtr), m1.data(), sizeof(float), sizeof(float), (size_t)R, cudaMemcpyHostToDevice, e->stream));
+    CK(cudaMemcpy2DAsync(field, sizeof(RepCtr), m1.data(), sizeof(float) * k, sizeof(float) * k, (size_t)R, cudaMemcpyHostToDevice, e->stream));
     CK(cudaStreamSynchronize(e->stream));
-    e->h2d_bytes += (int64_t)sizeof(float) * R;
+    e->h2d_bytes += (int64_t)sizeof(float) * k * R;
     return 0;
 }
 
-extern "C" int rb_read_transmission_scale(rb_engine *e, float *out) {
+static int read_replica_scales(rb_engine *e, const float *field, int k, float *out) {
     CK(cudaSetDevice(e->cfg.device));
     if (sync_all_streams(e)) return 1;
-    CK(cudaMemcpy2D(out, sizeof(float), &e->G.ctr[0].tscale_m1, sizeof(RepCtr), sizeof(float), (size_t)e->G.R, cudaMemcpyDeviceToHost));
-    for (int r = 0; r < e->G.R; r++) out[r] = 1.0f + out[r];
-    e->d2h_bytes += (int64_t)sizeof(float) * e->G.R;
+    CK(cudaMemcpy2D(out, sizeof(float) * k, field, sizeof(RepCtr), sizeof(float) * k, (size_t)e->G.R, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < e->G.R * k; i++) out[i] = 1.0f + out[i];
+    e->d2h_bytes += (int64_t)sizeof(float) * k * e->G.R;
     return 0;
+}
+
+extern "C" int rb_set_transmission_scale(rb_engine *e, const float *scale) {
+    return set_replica_scales(e, "rb_set_transmission_scale", &e->G.ctr[0].tscale_m1, 1, scale);
+}
+
+extern "C" int rb_read_transmission_scale(rb_engine *e, float *out) {
+    return read_replica_scales(e, &e->G.ctr[0].tscale_m1, 1, out);
+}
+
+extern "C" int rb_set_severity_scale(rb_engine *e, const float *scale) {
+    return set_replica_scales(e, "rb_set_severity_scale", e->G.ctr[0].sscale_m1, 3, scale);
+}
+
+extern "C" int rb_read_severity_scale(rb_engine *e, float *out) {
+    return read_replica_scales(e, e->G.ctr[0].sscale_m1, 3, out);
 }
 
 // ---------------------------------------------------------------- moving replicas between engines and GPUs (branch.cuh)

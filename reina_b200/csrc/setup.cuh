@@ -203,7 +203,7 @@ __global__ void k_sample(Eng G, uint32_t seed, int what, int age, int severity, 
             res = lo;
         } else if (what == 1) {
             u32x4 x = philox(seed, (uint32_t)i, (uint32_t)age, pu, 0);
-            res = symptom_severity(v, age, u01f(x.x), false);
+            res = symptom_severity(v, age, u01f(x.x), false, 0.0f, 0.0f, 0.0f);      // no replica: unscaled
         } else if (what == 2) {
             res = round_to_int(gamma_f(seed, (uint32_t)i, (uint32_t)age, pu, v->incubation_kappa, v->incubation_theta));
         } else {

@@ -134,6 +134,10 @@ struct RepCtr {
     // blobs and records of earlier builds load with f = 1, and every copy of a replica's counters carries f along.
     alignas(128) float tscale_m1;
     uint32_t reserved;
+    // the replica's severity scales minus 1: severe, critical, fatal (rb_set_severity_scale; symptom_severity scales the
+    // variant's conditional probabilities by 1 + sscale_m1 when device_infect draws an infection's severity).  Same line,
+    // same reasons: a zeroed RepCtr means 1, and every copy of the counters carries them.
+    float sscale_m1[3];
     // wide day boundary (boundary.cuh, Team): grid barrier word on its own line, today's verdict, per-CTA scan totals
     alignas(128) unsigned int wide_bar;
     alignas(128) uint32_t wide_day;
@@ -141,6 +145,10 @@ struct RepCtr {
     long long dbg_t[16];                          // measurement aid: cycles spent per phase of the day-boundary kernel
     long long dbg_last;
 };
+// rb_save_state and replica records store RepCtr raw, and the kernels' field offsets are as built: the scales above must
+// fit the padding of their line
+static_assert(sizeof(RepCtr) == 9728, "RepCtr layout changed: blobs and replica records of earlier builds would not load");
+static_assert(offsetof(RepCtr, wide_bar) == 8320, "RepCtr layout changed after the scales' line");
 
 struct Eng {
     int32_t dbg;                                   // measurement aid: 9 = the day-boundary kernels record cycles per phase (RepCtr::dbg_t)
@@ -251,19 +259,28 @@ __device__ __forceinline__ void mark_detected(const Eng &G, int r, int32_t a) {
 __device__ __forceinline__ void count_add(RepCtr *c, int attr, int age, int d) { atomicAdd(&c->counts[attr][age], d); }
 __device__ __forceinline__ void set_problem(RepCtr *c, int p) { atomicCAS(&c->problem, 0, p); }
 
-// Disease.get_symptom_severity, main.pyx:1042-1091 (every FATAL case dies outside hospital, SURVEY 8a note 2)
-__device__ __forceinline__ int symptom_severity(const rb_variant *v, int age, float val, bool vacc_eff) {
+// Disease.get_symptom_severity, main.pyx:1042-1091 (every FATAL case dies outside hospital, SURVEY 8a note 2).
+// s_m1, c_m1, q_m1: the replica's severity scales minus 1 (RepCtr::sscale_m1).  Each scaled probability is clamped to
+// max(x, 1), so it passes 1 only where the table already does, and at a scale of exactly 1 x * 1 == x and the clamp
+// returns x: bit for bit the unscaled draw.  The fatal scale acts on both fatal paths (fc and dohc).  dohc' = 1 makes
+// (val - dohc) / (1 - dohc) divide by zero, as the reference would: -inf (IEEE, -fmad=false), so the case is FATAL.
+__device__ __forceinline__ int symptom_severity(const rb_variant *v, int age, float val, bool vacc_eff, float s_m1, float c_m1,
+                                                float q_m1) {
     float vmod = 1.0f;
     if (vacc_eff) vmod = vmod * 0.1f;
     float syc = v->tab[RB_T_SYMPTOMATIC][age];
     if (val >= syc) return RB_ASYMPTOMATIC;
     syc = syc * vmod;
     float dohc = v->tab[RB_T_DEATH_OUTSIDE_HOSPITAL][age];
+    dohc = fminf(dohc * (1.0f + q_m1), fmaxf(dohc, 1.0f));
     if (dohc != 0.0f) {
         if (val < dohc * syc) return RB_FATAL;
         val = (val - dohc) / (1.0f - dohc);
     }
     float sc = v->tab[RB_T_SEVERE][age], cc = v->tab[RB_T_CRITICAL][age], fc = v->tab[RB_T_FATAL][age];
+    sc = fminf(sc * (1.0f + s_m1), fmaxf(sc, 1.0f));
+    cc = fminf(cc * (1.0f + c_m1), fmaxf(cc, 1.0f));
+    fc = fminf(fc * (1.0f + q_m1), fmaxf(fc, 1.0f));
     if (val < ((fc * cc) * sc) * syc) return RB_FATAL;
     if (val < (cc * sc) * syc) return RB_CRITICAL;
     if (val < sc * syc) return RB_SEVERE;
@@ -285,7 +302,8 @@ __device__ __forceinline__ void list_add(const Eng &G, int r, RepCtr *c, uint32_
 }
 
 // person_infect, main.pyx:209-235 + Population.infect :1576-1582.  `src_h` = packed word of the infector
-// (ignored when src < 0).  Severity and incubation use wild-type parameters (variant_idx is still 0 there).
+// (ignored when src < 0).  Severity and incubation use wild-type parameters (variant_idx is still 0 there); severity
+// with the replica's own severity scales (c is always &G.ctr[r], never a sharded message header).
 // `list`: the active list the new entry goes to (0 / 1), or -1 for none (the caller rebuilds the lists afterwards).
 __device__ void device_infect(const Eng &G, int r, RepCtr *c, int32_t t, int32_t src, uint32_t src_h, int variant,
                               int slot, bool fresh, int list, bool has_list) {
@@ -304,7 +322,7 @@ __device__ void device_infect(const Eng &G, int r, RepCtr *c, int32_t t, int32_t
     int sev = 0, dl = 0;
     if (owns(G, (uint32_t)t)) {     // severity and day counters are only ever read by the owner's sweep (sharded mode)
         u32x4 x = philox(c->seed, (uint32_t)t, (uint32_t)day, PU_SEVERITY, 0);
-        sev = symptom_severity(v0, age, u01f(x.x), vacc_eff);
+        sev = symptom_severity(v0, age, u01f(x.x), vacc_eff, c->sscale_m1[0], c->sscale_m1[1], c->sscale_m1[2]);
         dl = clamp255(round_to_int(gamma_f(c->seed, (uint32_t)t, (uint32_t)day, PU_INCUB, v0->incubation_kappa, v0->incubation_theta)));
     }
     if (src >= 0) {

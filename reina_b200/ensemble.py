@@ -351,19 +351,43 @@ def _move_replicas(ctxs, comm, rank, src, seeds, R):
         ctx.import_replicas(js % R, np.frombuffer(got[p], dtype=np.uint8).reshape(len(js), -1), seeds[js])
 
 
-def _set_scales(ctxs, rank, R, scale):
-    """Each of this process's Contexts sets its slice of the global scales (ctxs[i] holds global replicas (rank + i) R ..)."""
-    for i, c in enumerate(ctxs):
-        g0 = (rank + i) * R
-        c.set_transmission_scale(scale[g0:g0 + R])
-
-
-# the range a filtered transmission scale is kept in: the engine accepts (0, 16]
+# the range a filtered scale is kept in: the engine accepts (0, 16]
 _LOG_SCALE_MIN, _LOG_SCALE_MAX = math.log(1.0 / 16.0), math.log(16.0)
 
 
+class _FilteredScale:
+    """One per-replica log-scale parameter the particle filter estimates along with the state: the prior draw, the
+    scales each observation's weights judged, the resampling and the random-walk step, for every global replica.
+    `put(ctx, values)` sets one Context's slice (ctxs[i] holds global replicas (rank + i) R ..)."""
+
+    def __init__(self, what, prior, volatility, put, rng, N, n_days):
+        median, log_sd = (float(x) for x in prior)
+        if not (median > 0 and log_sd >= 0 and volatility >= 0):
+            raise ValueError('%s needs median > 0 and log_sd >= 0, and the volatility must be >= 0' % what)
+        self.volatility, self.put = volatility, put
+        self.log = np.clip(rng.normal(math.log(median), log_sd, N), _LOG_SCALE_MIN, _LOG_SCALE_MAX)
+        self.value = np.exp(self.log).astype(np.float32)
+        self.judged = np.zeros((n_days, N), dtype=np.float32)
+
+    def resample_and_step(self, src, rng, dt):
+        """Follow the resampling (the copies already carry their source's scale on the device), then take the step to
+        the next observation (dt days; None after the last).  True when the values changed and must be set."""
+        self.log, self.value = self.log[src], self.value[src]
+        if dt is None or self.volatility <= 0:
+            return False
+        self.log = np.clip(self.log + self.volatility * math.sqrt(dt) * rng.standard_normal(self.log.size),
+                           _LOG_SCALE_MIN, _LOG_SCALE_MAX)
+        self.value = np.exp(self.log).astype(np.float32)
+        return True
+
+    def set(self, ctxs, rank, R):
+        for i, c in enumerate(ctxs):
+            g0 = (rank + i) * R
+            self.put(c, self.value[g0:g0 + R])
+
+
 def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_threshold=0.5, seed=0, comm=None,
-                    transmission_prior=None, transmission_volatility=0.0):
+                    transmission_prior=None, transmission_volatility=0.0, severity_prior=None, severity_volatility=0.0):
     """Sequential importance resampling of an ensemble against observed counts: the replicas of ONE Context, of a list
     of Contexts of this process, or of every rank's Context (`comm`, one Context per rank), filtered as ONE set of
     particles.  Global replica g = k R + r is replica r of Context / rank k; every Context holds R replicas.
@@ -401,7 +425,16 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
     in [log 1/16, log 16].  After the last observation there is no step: the forecast runs with the scales in force.  The
     output then also holds transmission_scale[k, K R], the scales (float32, as set) the weights of day k judged:
     weighted_quantiles(out['transmission_scale'][k], out['weights'][k], q) is the scale's posterior band at that day.
-    With transmission_prior None, transmission_scale is None and the Contexts' scales are never touched."""
+    With transmission_prior None, transmission_scale is None and the Contexts' scales are never touched.
+
+    severity_prior = {name: (median, log_sd)} for any of model.SEVERITY_SCALES ('severe', 'critical', 'fatal') filters
+    those severity scales (Context.set_severity_scale) the same way, each with its own prior and the random-walk step
+    severity_volatility * sqrt(d_next - d) * eps.  They pin down what the transmission scale alone cannot: `severe` moves
+    in_ward, `critical` in_icu and `fatal` dead per infection, so together with all_detected the filter can tell more
+    infections from sicker ones.  The Generator draws the transmission scale first (prior and every step, exactly as
+    without severity_prior), then severe, critical and fatal, the named ones only; scales not named are never touched.
+    The output holds severity_scale = {name: [k, K R] float32}, the scales the weights of day k judged, for the named
+    scales; with severity_prior None it is None and no severity call is made."""
     ctxs = list(ctx) if isinstance(ctx, (list, tuple)) else [ctx]
     comm = comm or LocalComm()
     if not ctxs or (len(ctxs) > 1 and comm.size > 1):
@@ -419,16 +452,19 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
     out = dict(log_evidence=0.0, days=np.array(days, dtype=np.int64), ess=np.zeros(len(days)),
                resampled=np.zeros(len(days), dtype=bool), ancestors=np.zeros((len(days), N), dtype=np.int32),
                loglik=np.zeros((len(days), N)), seeds=np.zeros((len(days), N), dtype=np.uint32),
-               weights=np.zeros((len(days), N)), transmission_scale=None)
-    logf = None
+               weights=np.zeros((len(days), N)), transmission_scale=None, severity_scale=None)
+    if severity_prior is not None and (not severity_prior or set(severity_prior) - set(_model.SEVERITY_SCALES)):
+        raise ValueError('severity_prior: a dict over some of %s, not %r' % (_model.SEVERITY_SCALES, sorted(severity_prior)))
+    scales = {}                                       # transmission first, then severe, critical, fatal: the draw order
     if transmission_prior is not None:
-        median, log_sd = (float(x) for x in transmission_prior)
-        if not (median > 0 and log_sd >= 0 and transmission_volatility >= 0):
-            raise ValueError('transmission_prior needs median > 0 and log_sd >= 0, and the volatility must be >= 0')
-        logf = np.clip(rng.normal(math.log(median), log_sd, N), _LOG_SCALE_MIN, _LOG_SCALE_MAX)
-        scale = np.exp(logf).astype(np.float32)
-        _set_scales(ctxs, rank, R, scale)
-        out['transmission_scale'] = np.zeros((len(days), N), dtype=np.float32)
+        scales['transmission'] = _FilteredScale('transmission_prior', transmission_prior, transmission_volatility,
+                                                lambda c, v: c.set_transmission_scale(v), rng, N, len(days))
+    for name in _model.SEVERITY_SCALES:
+        if severity_prior is not None and name in severity_prior:
+            scales[name] = _FilteredScale('severity_prior[%r]' % name, severity_prior[name], severity_volatility,
+                                          lambda c, v, name=name: c.set_severity_scale(**{name: v}), rng, N, len(days))
+    for s in scales.values():
+        s.set(ctxs, rank, R)
     hist = None
     for k, d in enumerate(days):
         parts = []
@@ -455,8 +491,8 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
         w = np.exp(logw)
         ess = 1.0 / (w * w).sum()
         out['weights'][k] = w
-        if logf is not None:
-            out['transmission_scale'][k] = scale
+        for s in scales.values():
+            s.judged[k] = s.value
         src = np.arange(N, dtype=np.int32)
         if ess < ess_threshold * N or k == len(days) - 1:
             src = migration_plan(systematic_resample(w, rng), N // R)
@@ -471,13 +507,13 @@ def particle_filter(ctx, observations, *, model='negbin', dispersion=10.0, ess_t
             out['resampled'][k] = True
         out['ess'][k], out['ancestors'][k], out['loglik'][k] = ess, src, ll
         out['seeds'][k] = hist[:, d]
-        if logf is not None:
-            logf, scale = logf[src], scale[src]           # the copies already carry their source's scale on the device
-            if k < len(days) - 1 and transmission_volatility > 0:
-                step = transmission_volatility * math.sqrt(days[k + 1] - d)
-                logf = np.clip(logf + step * rng.standard_normal(N), _LOG_SCALE_MIN, _LOG_SCALE_MAX)
-                scale = np.exp(logf).astype(np.float32)
-                _set_scales(ctxs, rank, R, scale)
+        for s in scales.values():
+            if s.resample_and_step(src, rng, days[k + 1] - d if k < len(days) - 1 else None):
+                s.set(ctxs, rank, R)
+    if 'transmission' in scales:
+        out['transmission_scale'] = scales['transmission'].judged
+    if severity_prior is not None:
+        out['severity_scale'] = {n: scales[n].judged for n in _model.SEVERITY_SCALES if n in scales}
     return out
 
 

@@ -34,6 +34,9 @@ STATE_TO_STR = {0: 'SUSCEPTIBLE', 1: 'INCUBATION', 2: 'ILLNESS', 3: 'HOSPITALIZE
                 5: 'RECOVERED', 6: 'DEAD'}
 SEVERITY_TO_STR = {0: 'ASYMPTOMATIC', 1: 'MILD', 2: 'SEVERE', 3: 'CRITICAL', 4: 'FATAL'}
 STR_TO_SEVERITY = {v: k for k, v in SEVERITY_TO_STR.items()}
+# the columns of Context.set_severity_scale / severity_scale: the observed series each one mainly moves is in_ward,
+# in_icu and dead
+SEVERITY_SCALES = ('severe', 'critical', 'fatal')
 PROBLEM_TO_STR = {
     0: 'No problemos', 1: 'Too many infectees', 2: 'Too many contacts', 3: 'Hospital accounting failure',
     4: 'Negative number of contacts', 5: 'Malloc failure', 6: 'Other failure', 7: 'Wrong state',
@@ -683,6 +686,37 @@ class Context:
         """float32 [n_replicas]: the scales in force, as the engine applies them (1 + (f - 1) in float: f itself for
         0.5 <= f <= 2)."""
         return self._engine.read_transmission_scale()
+
+    def set_severity_scale(self, severe=None, critical=None, fatal=None):
+        """Every replica's severity scales (rb_set_severity_scale), column by column: each argument is None (keep the
+        scales in force), one value for all replicas or n_replicas values, each finite and in (0, 16].  Where an
+        infection's severity is drawn -- transmissions, imports and the initial state (rb_set_initial_state, which reads
+        the scales when it runs) -- the wild-type variant's conditional probabilities of the infected age become
+        min(x s, max(x, 1)): p_severe times `severe`, p_critical times `critical`, and both p_fatal and
+        p_death_outside_hospital times `fatal`, in force from the next iterate() on.  A scaled probability never passes 1
+        unless the table's already does, and a scale of 1 draws exactly as an unscaled Context does.  `severe` moves
+        in_ward, `critical` in_icu and `fatal` dead; FATAL is nested inside CRITICAL and every FATAL case dies outside
+        hospital, so raising `fatal` turns critical cases into deaths and in_icu falls.  sample('symptom_severity') stays
+        unscaled.  The scales are part of the replica's state: branch(), export / import, copy_replicas_from() and
+        save_state() / load_state() carry them, and reset() and a fresh Context give 1.  The full [n_replicas, 3] is
+        built from severity_scale() and the given columns and set in one engine call: refused values raise EngineError
+        and change nothing, the columns left as None included."""
+        R = self.n_replicas
+        s = self.severity_scale().astype(np.float64)
+        for j, values in enumerate((severe, critical, fatal)):
+            if values is None:
+                continue
+            v = np.full(R, values, dtype=np.float64) if np.ndim(values) == 0 else np.asarray(values, dtype=np.float64)
+            if v.shape != (R,):
+                raise ValueError('severity scale %s: one value or %d values' % (SEVERITY_SCALES[j], R))
+            s[:, j] = v
+        with np.errstate(over='ignore'):                  # a value beyond float32 becomes inf, which the engine refuses
+            self._engine.set_severity_scale(s.astype(np.float32))
+
+    def severity_scale(self):
+        """float32 [n_replicas, 3]: the severe, critical and fatal scales in force (SEVERITY_SCALES order), as the engine
+        applies them (1 + (s - 1) in float)."""
+        return self._engine.read_severity_scale()
 
     def row_layout(self):
         G = len(self.age_group_labels)
